@@ -3,6 +3,7 @@
 
     python bench.py --gpus 1 --steps K --warmup W          # this repo's sm_100a path
     python bench.py --impl reference ...                   # the reference's CPU path (oracle port) on host cores
+    python bench.py ... --dump-outputs DIR                 # also write the last timed step's outputs to DIR/*.npy
 
 One step = one pass of the hot path over one batch of synthetic middle slices:
 K1 normalise+resize -> ConvNeXt-base localizer -> K3 crops (128^2 + 256^2).  Workload (N=1):
@@ -34,6 +35,7 @@ SLICE_HW = (1195, 1195)
 TRAFFIC_JSON = os.environ.get("SVB_TRAFFIC_JSON", "r03z_gemm_traffic.json")  # per-shape DRAM bytes of the GEMM launches (ncu --set full), see scripts/summarise_ncu_layers.py
 WORKLOAD = ("configs[1]: 256 synthetic sagittal series per GPU (15x512x512 fp32 @0.7mm; middle plane at 0.3mm iso = 1195x1195), "
             "convnext_base random-init localizer @512x512, 5 IVD levels, crop_delta_mm 50/20/30/30, 128x128 crops + 256x256 classifier input")
+DUMP_SERIES = 32  # --dump-outputs: 32 series x 5 levels x (128^2 + 256^2) float32 = 52 MB per dump, whatever --batch is
 
 
 def workload_config(args):
@@ -60,7 +62,15 @@ def parse():
     ap.add_argument("--cpu-baseline-series", type=int, default=32,
                     help="series per pass of the cpu_baseline leg (N=1, rank 0): BASELINE configs[0]'s batch of 32, one warm-up + two timed passes = about 12 s of CPU work")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (rank 0) as float32 DIR/<name>.npy: coords "
+                         f"of every series, crops and crops2 of a fixed seeded sample of {DUMP_SERIES} series")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
+    return args
 
 
 # ----------------------------------------------------------------------------- CPU reference arm
@@ -135,6 +145,20 @@ def gpu_eager_rate(dev: str, batch: int = 64, reps: int = 5):
     del m, x
     torch.cuda.empty_cache()
     return batch / (ms * 1e-3), ms
+
+
+def dump_outputs(out_dir: str, batch) -> None:
+    """Write a pipeline.CropBatch as float32 .npy files (coords [B,5,2]; crops [S,5,128,128] and crops2 [S,5,256,256] of S =
+    min(B, DUMP_SERIES) series drawn with a fixed seed), so that two builds run with the same arguments compare output for output."""
+    import numpy as np
+    import torch
+
+    B = int(batch.coords.shape[0])
+    rows = np.sort(np.random.default_rng(0).choice(B, size=min(B, DUMP_SERIES), replace=False))
+    idx = torch.from_numpy(rows).to(batch.coords.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("coords", batch.coords), ("crops", batch.crops[idx]), ("crops2", batch.crops2[idx])):
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.float().cpu().numpy())
 
 
 # ----------------------------------------------------------------------------- clocks sampler
@@ -250,9 +274,12 @@ def run_b200(args):
     pool = series.resident_pool(dev)  # the isotropic middle slices of the batch, resident in HBM (K0 run once, outside the timed region)
     torch.cuda.synchronize()
 
+    last = {}
+
     def resident_step():
         b = step_resident(pool)
         gather(b.coords, b.crops)
+        last["batch"] = b
 
     for _ in range(args.warmup):
         resident_step()
@@ -261,6 +288,9 @@ def run_b200(args):
     _lib.load().svb_launch_count(1)
     ms_total = timed(resident_step, args.steps)
     gpu_launches = int(_lib.load().svb_launch_count(1))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["batch"])
+    del last["batch"]
     # roofline pass: same steps with a CUDA event pair around every launch of the model, and around
     # K1 / K3 with their (tiny) index tensors prebuilt so that no host work sits between the events
     times: dict = {}
