@@ -228,6 +228,11 @@ int svb_model_forward(svb_model* m, const uint8_t* d_in_u8, int B, int H, int W,
  * same code.  The dataset path does not use it (it feeds K1's uint8 plane to the folded stem). */
 int svb_model_forward_f32(svb_model* m, const float* d_in_nchw, int B, int H, int W, float* d_coords,
                           int micro_batch, void* d_ws, size_t ws_bytes, void* stream, float* times_ms);
+/* svb_model_forward (same kernels, micro-batches, streams and plans) that also reads out the residual stream after the last
+ * block of stages 0 .. n_stage_out - 1 (tests, profiling): d_stage_out[s] is a device buffer [B, H / 2^(s+2), W / 2^(s+2), dims[s]]
+ * of the model dtype, written by one device-to-device copy per micro-batch on the stream that computed it.  1 <= n_stage_out <= 4. */
+int svb_model_forward_stages(svb_model* m, const uint8_t* d_in_u8, int B, int H, int W, float* d_coords, int micro_batch,
+                             void* d_ws, size_t ws_bytes, void* stream, void* const* d_stage_out, int n_stage_out);
 /* model geometry: out[0]=num_levels, out[1]=num_outputs, out[2..5]=dims, out[6..9]=depths */
 int svb_model_info(const svb_model* m, int32_t out[10]);
 /* total tensor-core GEMM flops and launches of one forward over B images (for the roofline) */

@@ -1,89 +1,31 @@
-"""CPU emulation of the device numerics of the localizer (16-bit storage / GEMM operands, fp32 accumulation) to predict the
-coordinate error of a kernel design BEFORE building it.
+"""Predicted coordinate error of the device forward (16-bit storage / GEMM operands, fp32 accumulation) from its CPU
+emulation, ``oracle/emulate.py``, against the fp32 oracle, per stage and at the coordinates:
 
-    python scripts/emulate_precision.py [fp16|bf16]
+    python scripts/emulate_precision.py [fp16|bf16] [variant] [H W]
 
-Schemes per ConvNeXt block:
-  current   A = r16(LN(dwconv(x)));                           H = r16(gelu(A @ r16(W1)^T + b1))
-  ln_fold   y16 = r16(dwconv(x)); stats from y16;             H = r16(gelu(rstd * (y16 @ r16(W1 * g)^T - mu * s) + t))
-            (LayerNorm folded into fc1: s_n = sum_k r16(W1*g)[n,k], t = W1 @ b_ln + b1 -- the depthwise kernel then writes the raw
-             convolution and two statistics per token; no TMEM parking, no second pass)
-  tc_dw     ln_fold with the depthwise taps rounded to 16 bits (operands of the tensor-core depthwise kernel, dwconv_rawtc_kernel)
-  tc_dw_h   tc_dw with the off-centre column partial sums rounded to 16 bits before the cross-lane sum (packed shuffles)
 Test infrastructure (imports oracle/)."""
 import sys
 from pathlib import Path
 
-import numpy as np
 import torch
-import torch.nn.functional as F
 
 sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
+from oracle import emulate  # noqa: E402
 from oracle import reference_path as ref  # noqa: E402
 from oracle.convnext import make_model  # noqa: E402
 from spine_vision_b200 import synthetic  # noqa: E402
 
 DT = torch.float16 if (len(sys.argv) < 2 or sys.argv[1] == "fp16") else torch.bfloat16
-r16 = lambda t: t.to(DT).float()  # noqa: E731
+VARIANT = sys.argv[2] if len(sys.argv) > 2 else "base"
+SIZE = (int(sys.argv[3]), int(sys.argv[4])) if len(sys.argv) > 4 else (512, 512)
 torch.set_num_threads(8)
 
-
-def ln(x, w, b, eps=1e-6):
-    return F.layer_norm(x, (x.shape[-1],), w, b, eps)
-
-
-def forward(m, x, scheme):
-    bb = m.backbone
-    # stem (folded in the product; here: fp32 conv + LN, output stored in 16 bits)
-    x = bb.stem[0](x).permute(0, 2, 3, 1)
-    x = r16(ln(x, bb.stem[1].weight, bb.stem[1].bias))
-    for st in bb.stages:
-        if not isinstance(st.downsample, torch.nn.Identity):
-            a = r16(ln(x, st.downsample[0].weight, st.downsample[0].bias))
-            w = r16(st.downsample[1].weight)
-            x = r16(F.conv2d(a.permute(0, 3, 1, 2), w, st.downsample[1].bias, stride=2).permute(0, 2, 3, 1))
-        for blk in st.blocks:
-            wdw = r16(blk.conv_dw.weight) if scheme.startswith("tc_dw") else blk.conv_dw.weight  # tc_dw: taps are 16-bit tensor-core operands
-            if scheme == "tc_dw_h":
-                # the six off-centre stencil COLUMNS' partial sums (over the 7 rows) cross lanes as 16-bit values
-                xc = x.permute(0, 3, 1, 2)
-                y = blk.conv_dw.bias[None, :, None, None] + 0 * xc
-                for dx in range(7):
-                    wcol = torch.zeros_like(wdw)
-                    wcol[..., dx] = wdw[..., dx]
-                    part = F.conv2d(xc, wcol, None, padding=3, groups=x.shape[-1])
-                    y = y + (part if dx == 3 else r16(part))
-                y = y.permute(0, 2, 3, 1)
-            else:
-                y = F.conv2d(x.permute(0, 3, 1, 2), wdw, blk.conv_dw.bias, padding=3, groups=x.shape[-1]).permute(0, 2, 3, 1)
-            W1, b1 = blk.mlp.fc1.weight, blk.mlp.fc1.bias
-            if scheme == "current":  # (the round-1 block; not in the default list any more)
-                a = r16(ln(y, blk.norm.weight, blk.norm.bias))
-                h = a @ r16(W1).t() + b1
-            else:
-                y16 = r16(y)
-                mu = y16.mean(-1, keepdim=True)
-                var = (y16 * y16).mean(-1, keepdim=True) - mu * mu
-                rstd = torch.rsqrt(var + 1e-6)
-                Wg = r16(W1 * blk.norm.weight[None, :])
-                s = Wg.sum(1)
-                t = (W1.double() @ blk.norm.bias.double()).float() + b1
-                acc = y16 @ Wg.t()
-                h = rstd * acc + (-mu * rstd) * s + t
-            h = r16(F.gelu(h))
-            o = h @ r16(blk.mlp.fc2.weight).t() + blk.mlp.fc2.bias
-            x = r16(x + blk.gamma * o)
-    f = x.mean(dim=(1, 2))
-    f = ln(f, bb.head.norm.weight, bb.head.norm.bias)
-    return m.head(f).view(-1, 5, 2)
-
-
 SLICES = [(20, 1195, 1195), (21, 640, 650), (22, 900, 700), (23, 512, 512)]
+xs = torch.stack([ref.preprocess_slice(synthetic.make_iso_slice(*c), SIZE)[1] for c in SLICES])
 for trained in (False, True):
-    m = make_model("base", seed=0, trained_like=trained)
-    xs = torch.stack([ref.preprocess_slice(synthetic.make_iso_slice(*c), (512, 512))[1] for c in SLICES])
-    with torch.no_grad():
-        want = m(xs)
-        for scheme in ("ln_fold", "tc_dw", "tc_dw_h"):
-            got = forward(m, xs, scheme)
-            print(f"{DT} trained_like={trained} {scheme:8s}: max coordinate error {float((got - want).abs().max()) * 512:.4f} px at 512^2", flush=True)
+    m = make_model(VARIANT, seed=0, trained_like=trained)
+    want, want_st = emulate.oracle_stages(m, xs)
+    got, got_st = emulate.forward_stages(m, xs, DT)
+    rel = " ".join(f"{float((g - w).norm() / w.norm()):.2e}" for g, w in zip(got_st, want_st))
+    print(f"{DT} {VARIANT} {SIZE} trained_like={trained}: max coordinate error {float((got - want).abs().max()) * 512:.4f} px "
+          f"(normalised x 512); stage relative errors {rel}", flush=True)

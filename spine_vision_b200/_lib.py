@@ -26,6 +26,7 @@ EXPORTS = (
     "svb_k1_workspace_bytes", "svb_k1_normalize_resize", "svb_normalize_u8_workspace_bytes", "svb_normalize_u8",
     "svb_k3_workspace_bytes", "svb_k3_crop_resample", "svb_k3_crop_resample_rotated",
     "svb_model_create", "svb_model_destroy", "svb_model_workspace_bytes", "svb_model_forward", "svb_model_forward_f32",
+    "svb_model_forward_stages",
     "svb_model_info", "svb_model_cost", "svb_gemm", "svb_mlp_fused", "svb_mlp_fused_ln",
     "svb_stem_ln", "svb_dwconv_ln", "svb_dwconv_raw", "svb_dwconv_tc_pack", "svb_dwconv_raw_tc", "svb_dwconv_ln_tc", "svb_ln_patchify", "svb_head",
     "svb_k4_classifier_input",
@@ -114,6 +115,8 @@ def load() -> C.CDLL:
     lib.svb_model_forward.argtypes = [vp, vp, i32, i32, i32, vp, i32, vp, sz, vp, vp]
     lib.svb_model_forward_f32.restype = C.c_int
     lib.svb_model_forward_f32.argtypes = [vp, vp, i32, i32, i32, vp, i32, vp, sz, vp, vp]
+    lib.svb_model_forward_stages.restype = C.c_int
+    lib.svb_model_forward_stages.argtypes = [vp, vp, i32, i32, i32, vp, i32, vp, sz, vp, C.POINTER(vp), i32]
     lib.svb_model_info.restype = C.c_int
     lib.svb_model_info.argtypes = [vp, C.POINTER(C.c_int32 * 10)]
     lib.svb_model_cost.restype = C.c_int

@@ -221,6 +221,15 @@ class LocalizationModel:
     def predict_u8(self, planes_u8: torch.Tensor, times: dict | None = None, out: torch.Tensor | None = None) -> torch.Tensor:
         return self.engine.forward(planes_u8, times, out)
 
+    def predict_u8_stages(self, planes_u8: torch.Tensor) -> tuple[torch.Tensor, list[torch.Tensor]]:
+        """``predict_u8`` plus the residual stream after each of the four stages, ``[B, H / 2^(s+2), W / 2^(s+2), C_s]`` in the
+        model's 16-bit dtype (stage-level parity tests and profiling)."""
+        e = self.engine
+        B, H, W = planes_u8.shape
+        dt = torch.float16 if e.dtype in ("fp16", "float16", "half") else torch.bfloat16
+        stages = [torch.empty((B, H >> (s + 2), W >> (s + 2), e.dims[s]), dtype=dt, device=planes_u8.device) for s in range(4)]
+        return e.forward(planes_u8, stage_out=stages), stages
+
     def forward(self, x: torch.Tensor) -> torch.Tensor:
         """``CoordinateRegressor.forward`` (generic.py:380-391) for callers that build the input themselves:
         ``x`` = ``[B,3,H,W]`` float, /255 and ImageNet-normalised (any device / float dtype) -> ``[B, num_levels, 2]`` float32

@@ -1150,13 +1150,19 @@ struct Timer {  // optional per-launch CUDA-event timing, accumulated per kernel
 
 template <typename T>
 static int forward_chunk(svb_model* m, const uint8_t* in, const float* in_f32, int nb, int H, int W, float* coords, uint8_t* ws,
-                         cudaStream_t st, Timer& tm) {
+                         cudaStream_t st, Timer& tm, void* const* stage_out, int n_stage_out) {
     ActPlan* plan = nullptr;
     if (int rc = get_plan(m, ws, nb, H, W, &plan)) return rc;
     const WsLayout L = ws_layout(m, nb, H, W);
     T* X = reinterpret_cast<T*>(ws + L.x);
     T* A = reinterpret_cast<T*>(ws + L.a);
     T* Hd = reinterpret_cast<T*>(ws + L.h);
+    // svb_model_forward_stages: the residual stream after the last block of stage s, this micro-batch's images, on its own stream
+    auto stage_done = [&](int s, int h, int w) -> int {
+        if (s < n_stage_out)
+            SVB_CUDA_OK(cudaMemcpyAsync(stage_out[s], X, (size_t)nb * h * w * m->dims[s] * sizeof(T), cudaMemcpyDeviceToDevice, st));
+        return SVB_OK;
+    };
 #define RUN(cls, call)                             \
     {                                              \
         if (int rc = tm.begin(cls)) return rc;     \
@@ -1229,6 +1235,7 @@ static int forward_chunk(svb_model* m, const uint8_t* in, const float* in_f32, i
                                                     GEMM_RESID, st, false, nullptr, m0));
                 }
             }
+            if (int rc = stage_done(s, h, w)) return rc;
             continue;
         }
         for (const BlockParams& bp : m->blocks[s]) {
@@ -1248,6 +1255,7 @@ static int forward_chunk(svb_model* m, const uint8_t* in, const float* in_f32, i
                                                 GEMM_RESID, st, coex_stage(s)));
             }
         }
+        if (int rc = stage_done(s, h, w)) return rc;
     }
     {
         const int C = m->dims[3];
@@ -1280,7 +1288,8 @@ extern "C" size_t svb_model_workspace_bytes(const svb_model* m, int micro_batch,
 }
 
 static int model_forward_any(svb_model* m, const uint8_t* d_in_u8, const float* d_in_f32, int B, int H, int W, float* d_coords,
-                             int micro_batch, void* d_ws, size_t ws_bytes, void* stream_, float* times_ms) {
+                             int micro_batch, void* d_ws, size_t ws_bytes, void* stream_, float* times_ms,
+                             void* const* stage_out = nullptr, int n_stage_out = 0) {
     cudaStream_t st = static_cast<cudaStream_t>(stream_);
     SVB_REQUIRE(m && (d_in_u8 || d_in_f32) && d_coords && d_ws, SVB_ERR_INVALID_ARG, "model_forward: null argument");
     SVB_REQUIRE(B >= 0 && micro_batch > 0, SVB_ERR_INVALID_ARG, "model_forward: B=%d micro_batch=%d", B, micro_batch);
@@ -1306,10 +1315,13 @@ static int model_forward_any(svb_model* m, const uint8_t* d_in_u8, const float* 
         int rc;
         const uint8_t* in8 = d_in_u8 ? d_in_u8 + (size_t)b0 * H * W : nullptr;
         const float* in32 = d_in_f32 ? d_in_f32 + (size_t)b0 * 3 * H * W : nullptr;
+        void* so[4] = {};
+        for (int s = 0; s < n_stage_out; ++s)  // [B, H / 2^(s+2), W / 2^(s+2), C_s], 16-bit: this chunk starts at image b0
+            so[s] = static_cast<uint8_t*>(stage_out[s]) + (size_t)b0 * (H >> (s + 2)) * (W >> (s + 2)) * m->dims[s] * 2;
         if (m->dtype == SVB_FP16)
-            rc = forward_chunk<__half>(m, in8, in32, nb, H, W, d_coords + (size_t)b0 * m->nout, ws, cs, tm);
+            rc = forward_chunk<__half>(m, in8, in32, nb, H, W, d_coords + (size_t)b0 * m->nout, ws, cs, tm, so, n_stage_out);
         else
-            rc = forward_chunk<__nv_bfloat16>(m, in8, in32, nb, H, W, d_coords + (size_t)b0 * m->nout, ws, cs, tm);
+            rc = forward_chunk<__nv_bfloat16>(m, in8, in32, nb, H, W, d_coords + (size_t)b0 * m->nout, ws, cs, tm, so, n_stage_out);
         if (rc) return rc;
     }
     if (dual) {
@@ -1323,6 +1335,15 @@ extern "C" int svb_model_forward(svb_model* m, const uint8_t* d_in_u8, int B, in
                                  int micro_batch, void* d_ws, size_t ws_bytes, void* stream_, float* times_ms) {
     SVB_REQUIRE(d_in_u8, SVB_ERR_INVALID_ARG, "model_forward: null argument");
     return model_forward_any(m, d_in_u8, nullptr, B, H, W, d_coords, micro_batch, d_ws, ws_bytes, stream_, times_ms);
+}
+
+extern "C" int svb_model_forward_stages(svb_model* m, const uint8_t* d_in_u8, int B, int H, int W, float* d_coords, int micro_batch,
+                                        void* d_ws, size_t ws_bytes, void* stream_, void* const* d_stage_out, int n_stage_out) {
+    SVB_REQUIRE(d_in_u8 && d_stage_out, SVB_ERR_INVALID_ARG, "model_forward_stages: null argument");
+    SVB_REQUIRE(n_stage_out >= 1 && n_stage_out <= 4, SVB_ERR_INVALID_ARG, "model_forward_stages: %d stage buffers (1..4)", n_stage_out);
+    for (int s = 0; s < n_stage_out; ++s)
+        SVB_REQUIRE(d_stage_out[s], SVB_ERR_INVALID_ARG, "model_forward_stages: stage buffer %d is null", s);
+    return model_forward_any(m, d_in_u8, nullptr, B, H, W, d_coords, micro_batch, d_ws, ws_bytes, stream_, nullptr, d_stage_out, n_stage_out);
 }
 
 extern "C" int svb_model_forward_f32(svb_model* m, const float* d_in_nchw, int B, int H, int W, float* d_coords,

@@ -373,8 +373,11 @@ class LocalizationEngine:
         return fl.value, n.value
 
     @_on_device
-    def forward(self, u8: torch.Tensor, times: dict | None = None, out: torch.Tensor | None = None) -> torch.Tensor:
-        """uint8 [B,H,W] on the device -> float32 [B, num_levels, 2] in [0,1]."""
+    def forward(self, u8: torch.Tensor, times: dict | None = None, out: torch.Tensor | None = None,
+                stage_out: list[torch.Tensor] | None = None) -> torch.Tensor:
+        """uint8 [B,H,W] on the device -> float32 [B, num_levels, 2] in [0,1].  ``stage_out`` (tests, profiling): up to four
+        device tensors ``[B, H / 2^(s+2), W / 2^(s+2), dims[s]]`` of the model dtype that receive the residual stream after the
+        last block of stage s (``svb_model_forward_stages``: the same kernels and schedule as without it)."""
         assert u8.is_cuda and u8.dtype == torch.uint8 and u8.dim() == 3 and u8.is_contiguous()
         lib = _lib.load()
         B, H, W = u8.shape
@@ -386,6 +389,16 @@ class LocalizationEngine:
         need = lib.svb_model_workspace_bytes(self._h, mb, H, W)
         ws = _Workspace.get("model", need, u8.device)
         wp, wn = _aligned_ptr(ws, 1024)
+        if stage_out is not None:
+            assert times is None, "per-stage readout is not timed"
+            want = torch.float16 if _lib.DTYPES[self.dtype] == _lib.SVB_FP16 else torch.bfloat16
+            for s, t in enumerate(stage_out):
+                assert t.device == u8.device and t.dtype == want and t.is_contiguous(), f"stage {s}: {want} on {u8.device}"
+                assert tuple(t.shape) == (B, H >> (s + 2), W >> (s + 2), self.dims[s]), f"stage {s}: shape {tuple(t.shape)}"
+            ptrs = (C.c_void_p * len(stage_out))(*[t.data_ptr() for t in stage_out])
+            _lib.check(lib.svb_model_forward_stages(self._h, u8.data_ptr(), B, H, W, coords.data_ptr(), mb, wp, wn, _lib.current_stream(),
+                                                    ptrs, len(stage_out)))
+            return coords
         tbuf = (C.c_float * len(_lib.KERNEL_CLASSES))() if times is not None else None
         _lib.check(lib.svb_model_forward(self._h, u8.data_ptr(), B, H, W, coords.data_ptr(), mb, wp, wn, _lib.current_stream(),
                                          C.cast(tbuf, C.c_void_p) if tbuf is not None else None))

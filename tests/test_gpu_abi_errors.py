@@ -72,3 +72,30 @@ def test_model_create_rejects_incomplete_or_unsupported_checkpoints():
         eng.forward(torch.zeros((1, 500, 512), dtype=torch.uint8, device=dev()))  # H not a multiple of 32
     out = eng.forward(torch.zeros((0, 512, 512), dtype=torch.uint8, device=dev()))
     assert tuple(out.shape) == (0, 5, 2)
+
+
+@requires_gpu
+def test_model_forward_stages_rejects_bad_stage_buffers():
+    lib = _lib.load()
+    eng = ops.LocalizationEngine(synthetic.random_state_dict("tiny", seed=0), dev(), "fp16", micro_batch=2)
+    u8 = torch.zeros((3, 64, 64), dtype=torch.uint8, device=dev())
+    coords = torch.zeros((3, 5, 2), dtype=torch.float32, device=dev())
+    ws = torch.zeros(lib.svb_model_workspace_bytes(eng._h, 2, 64, 64) + 1024, dtype=torch.uint8, device=dev())
+    wp = (ws.data_ptr() + 1023) // 1024 * 1024
+    stages = [torch.zeros((3, 64 >> (s + 2), 64 >> (s + 2), eng.dims[s]), dtype=torch.float16, device=dev()) for s in range(4)]
+    st = torch.cuda.current_stream().cuda_stream
+
+    def call(bufs, n):
+        arr = (C.c_void_p * max(1, len(bufs)))(*bufs) if bufs else None
+        return lib.svb_model_forward_stages(eng._h, u8.data_ptr(), 3, 64, 64, coords.data_ptr(), 2, wp, ws.numel() - 1024, st, arr, n)
+
+    ptrs = [t.data_ptr() for t in stages]
+    assert call([], 4) == INVALID and "null" in _err()
+    assert call(ptrs, 0) == INVALID and "stage buffers" in _err()
+    assert call(ptrs, 5) == INVALID and "stage buffers" in _err()
+    assert call(ptrs[:2] + [None] + ptrs[3:], 4) == INVALID and "stage buffer 2 is null" in _err()
+    assert call(ptrs[:2], 2) == 0  # the first stages only
+    torch.cuda.synchronize()
+    assert stages[1].abs().sum() > 0 and stages[2].abs().sum() == 0
+    with pytest.raises(AssertionError):  # wrong shape caught before the call
+        eng.forward(u8, stage_out=[stages[1]])

@@ -4,7 +4,7 @@ import pytest
 import torch
 
 from conftest import GOLDEN
-from gpu_util import dev
+from gpu_util import dev, trained_like_gate
 from oracle import reference_path as ref
 from oracle.convnext import make_model
 from spine_vision_b200 import cropping, ops, pipeline, synthetic
@@ -246,7 +246,9 @@ def test_streamed_driver_equals_resident_path():
 @pytest.mark.parametrize("image_size", [(768, 768), (512, 768), (640, 384)])
 def test_model_other_input_sizes_config5(image_size):
     """BASELINE config 5 runs the localizer at 768x768; image_size is a config field (config.py:53-54), so any multiple
-    of 32 must work, square or not.  Same normalised tolerance as the 512^2 gate (0.5 px / 512)."""
+    of 32 must work, square or not.  Same normalised tolerance as the 512^2 gate (0.5 px / 512).  The random-init weights
+    (layer scale 1e-6) test the stem, the downsample layers and the head; the trained-like fp16 row, gated by what the emulation
+    of the device numerics predicts for the size, tests the ConvNeXt blocks."""
     om = make_model("base", seed=0)
     slices = [synthetic.make_iso_slice(50, 1195, 1195), synthetic.make_iso_slice(51, 700, 900)]
     want = []
@@ -265,6 +267,12 @@ def test_model_other_input_sizes_config5(image_size):
     err = np.abs(got - want).max()
     print(f"[coords] image_size={image_size}: max normalised error {err:.2e} ({err * 512:.3f} px at 512)")
     assert err <= 0.5 / 512
+    tm = make_model("base", seed=0, trained_like=True)
+    want_t, pred, gate = trained_like_gate(tm, torch.stack([ref.preprocess_slice(sl, image_size)[1] for sl in slices]))
+    got_t = cropping.LocalizationModel(tm.state_dict(), dev(), dtype="fp16").predict_u8(planes).cpu().numpy()
+    err_t = np.abs(got_t - want_t).max() * PX
+    print(f"[coords] image_size={image_size} trained-like fp16: {err_t:.4f} px (x 512), emulator predicts {pred:.4f}, gate {gate:.3f}")
+    assert err_t <= gate
 
 
 def test_config3_ragged_volumes_with_their_own_spacing():
@@ -335,7 +343,9 @@ def test_model_config5_scale_768_batch():
                                           ("small", (96, 192, 384, 768)), ("tiny", (96, 192, 384, 768))])
 def test_model_other_variants(variant, dims):
     """config.model_variant (config.py:27-39) beyond "base": every other ConvNeXt-v1 size -- tiny / small (96-channel stem: one
-    and a half 64-channel chunks), large (multiples of 64 only), xlarge.  Same gate as base: 0.5 px at 512^2 vs the fp32 oracle."""
+    and a half 64-channel chunks), large (multiples of 64 only), xlarge.  Same gate as base: 0.5 px at 512^2 vs the fp32 oracle.
+    Random-init weights (layer scale 1e-6) hide every block, so they test the stem, the downsample layers and the head at these
+    widths; the trained-like fp16 row tests the blocks, gated by what the emulation of the device numerics predicts."""
     om = make_model(variant, seed=0)
     slices = [synthetic.make_iso_slice(80, 700, 640), synthetic.make_iso_slice(81, 512, 512)]
     want = _oracle_coords(om, slices)
@@ -346,6 +356,12 @@ def test_model_other_variants(variant, dims):
     err_px = np.abs(got - want).max() * PX
     print(f"[coords] {variant} bf16: max error {err_px:.4f} px")
     assert np.isfinite(got).all() and err_px <= 0.5
+    tm = make_model(variant, seed=0, trained_like=True)
+    want_t, pred, gate = trained_like_gate(tm, torch.stack([ref.preprocess_slice(sl, (512, 512))[1] for sl in slices]))
+    got_t = cropping.LocalizationModel(tm.state_dict(), dev(), dtype="fp16").predict_u8(ops.normalize_resize(pool, (512, 512))).cpu().numpy()
+    err_t = np.abs(got_t - want_t).max() * PX
+    print(f"[coords] {variant} trained-like fp16: max error {err_t:.4f} px, emulator predicts {pred:.4f} px, gate {gate:.3f} px")
+    assert np.isfinite(got_t).all() and err_t <= gate
 
 
 @pytest.mark.parametrize("variant,dims,tol_px", [("v2_base", (128, 256, 512, 1024), 0.5), ("v2_tiny", (96, 192, 384, 768), 0.5),

@@ -7,7 +7,7 @@ import pytest
 import torch
 from PIL import Image
 
-from gpu_util import dev
+from gpu_util import dev, trained_like_gate
 from oracle import fixedpoint as fx
 from oracle import reference_path as ref
 from spine_vision_b200 import cropping, ops, synthetic
@@ -148,7 +148,10 @@ def test_k3_random_rotated_vs_reference(seed):
 @pytest.mark.parametrize("image_size", [(32, 32), (64, 32), (32, 96), (96, 160), (224, 224), (352, 288), (1024, 512)])
 def test_localizer_unusual_image_sizes_vs_fp32_oracle(image_size):
     """``image_size`` is a config field (config.py:53-54): every multiple of 32 must work, down to 32 x 32 where the last stage
-    is a single token and every depthwise window hangs over all four borders.  Same normalised gate as at 512^2 (0.5 px / 512)."""
+    is a single token and every depthwise window hangs over all four borders.  Same normalised gate as at 512^2 (0.5 px / 512).
+    Random-init weights (layer scale 1e-6) test the stem, the downsample layers and the head; the trained-like fp16 row tests the
+    ConvNeXt blocks (depthwise windows over the borders, tensor-core depthwise modes A and B), gated by what the emulation of the
+    device numerics predicts for the size."""
     from oracle.convnext import make_model
 
     om = make_model("base", seed=0)
@@ -166,6 +169,12 @@ def test_localizer_unusual_image_sizes_vs_fp32_oracle(image_size):
     err = float(np.abs(got - np.stack(want)).max())
     print(f"[coords] image_size={image_size}: max normalised error {err:.2e}")
     assert np.isfinite(got).all() and err <= 0.5 / 512
+    tm = make_model("base", seed=0, trained_like=True)
+    want_t, pred, gate = trained_like_gate(tm, torch.stack([ref.preprocess_slice(sl, image_size)[1] for sl in slices]))
+    got_t = cropping.LocalizationModel(tm.state_dict(), dev(), dtype="fp16", micro_batch=2).predict_u8(planes).cpu().numpy()
+    err_t = float(np.abs(got_t - want_t).max()) * 512
+    print(f"[coords] image_size={image_size} trained-like fp16: {err_t:.4f} px (x 512), emulator predicts {pred:.4f}, gate {gate:.3f}")
+    assert np.isfinite(got_t).all() and err_t <= gate
 
 
 def _k0_random_cases(seed, n):
