@@ -194,7 +194,10 @@ int svb_k3_crop_resample_rotated(const float* d_slices, const int64_t* d_offs, c
  * svb_model_create takes the checkpoint's "model_state_dict" (load_localization_model,
  * cropping.py:436-437) as an array of HOST fp32 tensors under their state-dict names; it
  * folds /255 + ImageNet mean/std + RGB replication into the 4x4 stem, repacks the weights
- * for the tensor-core kernels and uploads them.
+ * for the tensor-core kernels and uploads them.  Supported: stage widths that are multiples of 32
+ * in [96, 2816] and stem widths 96 / 128 / 192 / 256 / 352, i.e. every model_variant (tiny, small,
+ * base, large, xlarge, v2_tiny .. v2_large, and v2_huge: 352 / 704 / 1408 / 2816); anything else is
+ * SVB_ERR_UNSUPPORTED_MODEL.  With SVB_LN_FOLD=0 (the un-folded LayerNorm block) v2_huge is refused.
  */
 typedef struct svb_model svb_model;
 
@@ -259,9 +262,9 @@ int svb_mlp_fused_ln(const void* d_a, const void* d_w1g, const float* d_t, const
 /* ------------------------------------------------------------------------------------------
  * Standalone layer entries (unit tests / ncu captures of one kernel).  Same kernels the model runs.
  * x/out are NHWC 16-bit of `dtype`.
- *  svb_stem_ln     : u8 [B,H,W] -> [B,H/4,W/4,C0]; wf [C0][16], bf [C0] are the FOLDED stem (fp32)
+ *  svb_stem_ln     : u8 [B,H,W] -> [B,H/4,W/4,C0]; wf [C0][16], bf [C0] are the FOLDED stem (fp32); C0 = 96/128/192/256/352
  *  svb_dwconv_ln   : depthwise 7x7 (taps [49][C] fp32, tap-major) + bias + LayerNorm(C) eps 1e-6
- *  svb_ln_patchify : LayerNorm2d + 2x2/s2 gather -> [B,H/2,W/2,4C]
+ *  svb_ln_patchify : LayerNorm2d + 2x2/s2 gather -> [B,H/2,W/2,4C]; C = the stage-0..2 widths (96..1024, 352/704/1408)
  *  svb_head        : avg-pool over `tokens` + LayerNorm(eps 1e-6) + LayerNorm(eps 1e-5)
  *                    + Linear(C,HID) + GELU + Linear(HID,NOUT) + sigmoid -> coords fp32 [B,NOUT]
  */

@@ -250,8 +250,6 @@ def load_localization_model(model_path: Path, variant: str, device: str, dtype: 
     """cropping.py:407-441 -- same checkpoint format (``torch.save`` dict whose
     ``"model_state_dict"`` holds the 348 ``backbone.*`` / ``head.*`` tensors,
     trainers/base.py:695-706), strict key check, weights repacked for the tensor cores."""
-    if variant == "v2_huge":
-        raise NotImplementedError("convnextv2_huge (2816 channels) is beyond the depthwise kernel's 2048-channel limit")
     checkpoint = torch.load(model_path, map_location="cpu", weights_only=False)
     return LocalizationModel(checkpoint["model_state_dict"], device, dtype)
 

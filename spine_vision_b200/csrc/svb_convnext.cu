@@ -367,17 +367,26 @@ extern "C" int svb_model_create(svb_model** out, const svb_weight_desc* weights,
         const svb_weight_desc* g = hwts.get("backbone.stages." + std::to_string(s) + ".blocks.0.norm.weight");
         SVB_REQUIRE(g != nullptr, SVB_ERR_MISSING_WEIGHT, "model_create: state dict has no 'backbone.stages.%d.blocks.0.norm.weight'", s);
         m->dims[s] = (int)g->shape[0];
-        SVB_REQUIRE(m->dims[s] % 32 == 0 && m->dims[s] >= 96 && m->dims[s] <= 2048, SVB_ERR_UNSUPPORTED_MODEL,
-                    "stage %d width %d: this build supports the ConvNeXt-v1 widths (tiny / small 96..768, base 128..1024, "
-                    "large 192..1536, xlarge 256..2048)", s, m->dims[s]);
+        SVB_REQUIRE(m->dims[s] % 32 == 0 && m->dims[s] >= 96 && m->dims[s] <= 2816, SVB_ERR_UNSUPPORTED_MODEL,
+                    "stage %d width %d: this build supports the ConvNeXt widths (tiny / small 96..768, base 128..1024, "
+                    "large 192..1536, xlarge 256..2048, v2_huge 352..2816)", s, m->dims[s]);
     }
     SVB_REQUIRE(m->dims[0] == (int)stem_w->shape[0], SVB_ERR_UNSUPPORTED_MODEL, "stem width != stage-0 width");
     m->v2 = hwts.get("backbone.stages.0.blocks.0.mlp.grn.weight") != nullptr;  // timm convnextv2_*: GRN instead of layer scale
     m->ln_fold = ln_fold_env();
     m->tc2_setting = dw_tc2_env();
     m->mlp_fused_setting = mlp_fused_env();
-    SVB_REQUIRE(m->dims[0] == 96 || m->dims[0] == 128 || m->dims[0] == 192 || m->dims[0] == 256, SVB_ERR_UNSUPPORTED_MODEL,
-                "stem width %d unsupported", m->dims[0]);
+    SVB_REQUIRE(m->dims[0] == 96 || m->dims[0] == 128 || m->dims[0] == 192 || m->dims[0] == 256 || m->dims[0] == 352,
+                SVB_ERR_UNSUPPORTED_MODEL, "stem width %d unsupported (supported: 96 tiny / small, 128 base, 192 large, 256 xlarge, "
+                "352 v2_huge)", m->dims[0]);
+    // the un-folded block (SVB_LN_FOLD=0) runs dwconv_ln_kernel, which parks all channels in TMEM and has no instance at the
+    // convnextv2_huge widths: refuse such a model here rather than partway through a forward
+    for (int s = 0; s < 4 && !m->ln_fold; ++s) {
+        const int C = m->dims[s];
+        SVB_REQUIRE(C == 96 || C == 128 || C == 192 || C == 256 || C == 384 || C == 512 || C == 768 || C == 1024 || C == 1536 || C == 2048,
+                    SVB_ERR_UNSUPPORTED_MODEL, "stage %d width %d: SVB_LN_FOLD=0 (the un-folded LayerNorm block) does not support "
+                    "this width; unset it to run v2_huge", s, C);
+    }
     NEED(head_w1, "head.2.weight");
     NEED(head_w2, "head.5.weight");
     m->hid = (int)head_w1->shape[0];
@@ -631,8 +640,12 @@ static WsLayout ws_layout(const svb_model* m, int nb, int H, int W) {
     L.a = o; o += align_up(t0 * c0 * 2, 1024);
     L.h = o; o += align_up(t0 * c0 * 4 * 2, 1024);
     L.stat = o; o += align_up(t0 * 8, 1024);  // (rstd, -mu rstd) per token: the folded LayerNorm of the current block
-    // dwconv_rawtc_kernel's per-chunk partial (sum, sum of squares) [token][C / 64] (tokens x chunks is largest in stage 0)
-    L.stat_part = o; o += align_up(t0 * 8 * std::max<size_t>(1, c0 / 64), 1024);
+    // dwconv_rawtc_kernel's per-chunk partial (sum, sum of squares) [token][C / 64]: the largest stage (stage 0 for every
+    // variant, but 352 / 64 floors to 5 chunks there, so it is not taken for granted)
+    size_t part_words = 0;
+    for (int s = 0, hs = H / 4, wsz = W / 4; s < 4; ++s, hs /= 2, wsz /= 2)
+        part_words = std::max(part_words, (size_t)nb * hs * wsz * std::max<size_t>(1, (size_t)m->dims[s] / 64));
+    L.stat_part = o; o += align_up(part_words * 8, 1024);
     L.grn_part = L.grn_scale = o;
     if (m->v2) {  // partial sums of squares [nb][ceil(tokens / GRN_ROWS)][4C] and scales [nb][4C]: the largest stage of each
         size_t part = 0, scale = 0;
@@ -980,10 +993,14 @@ static int launch_dwconv_rawtc(const CUtensorMap& x, const BlockParams& bp, void
 
 // rows per tile: 8, or 4 when 8-row tiles would leave most of the 2 x 148 CTA slots empty (the last stage: 16 x 16 tokens per image)
 static int dw_raw_th(int nb, int H, int W) { return nb * ceil_div(W, 16) * ceil_div(H, 8) >= num_sms() * 3 / 2 ? 8 : 4; }
+// 704, 1408 and 2816 channels (convnextv2_huge stages 1-3) take TH = 4 always: at TH = 8 they need more than the 128 registers of two CTAs
+// per SM and spill (44 B of stores, 80 B of loads per thread under ptxas 12.9)
 template <typename T, int C>
 static int launch_dwconv_raw_t(const CUtensorMap& x8, const CUtensorMap& x4, const BlockParams& bp, void* out, float2* rowstat, int nb, int H, int W,
                                cudaStream_t st, int b0) {
-    if (dw_raw_th(nb, H, W) == 8) return launch_dwconv_raw_th<T, C, 8>(x8, bp, out, rowstat, nb, H, W, st, b0);
+    constexpr bool th8_spills = C == 704 || C == 1408 || C == 2816;
+    if constexpr (!th8_spills)
+        if (dw_raw_th(nb, H, W) == 8) return launch_dwconv_raw_th<T, C, 8>(x8, bp, out, rowstat, nb, H, W, st, b0);
     return launch_dwconv_raw_th<T, C, 4>(x4, bp, out, rowstat, nb, H, W, st, b0);
 }
 template <typename T>
@@ -1000,6 +1017,10 @@ static int launch_dwconv_raw(const CUtensorMap& x, const CUtensorMap& x4, const 
         case 384: return launch_dwconv_raw_t<T, 384>(x, x4, bp, out, rowstat, nb, H, W, st, b0);
         case 768: return launch_dwconv_raw_t<T, 768>(x, x4, bp, out, rowstat, nb, H, W, st, b0);
         case 1536: return launch_dwconv_raw_t<T, 1536>(x, x4, bp, out, rowstat, nb, H, W, st, b0);
+        case 352: return launch_dwconv_raw_t<T, 352>(x, x4, bp, out, rowstat, nb, H, W, st, b0);  // convnextv2_huge
+        case 704: return launch_dwconv_raw_t<T, 704>(x, x4, bp, out, rowstat, nb, H, W, st, b0);
+        case 1408: return launch_dwconv_raw_t<T, 1408>(x, x4, bp, out, rowstat, nb, H, W, st, b0);
+        case 2816: return launch_dwconv_raw_t<T, 2816>(x, x4, bp, out, rowstat, nb, H, W, st, b0);
     }
     return set_error(SVB_ERR_UNSUPPORTED_MODEL, "dwconv (raw): unsupported width %d", C);
 }
@@ -1047,7 +1068,7 @@ static int launch_dwconv(const CUtensorMap& x, const BlockParams& bp, void* out,
 }
 template <typename T>
 static int launch_ln_patchify(const void* x, const DownParams& d, void* a2, int Cin, int nb, int H, int W, cudaStream_t st) {
-    const int pg = Cin <= 512 ? 4 : 2;  // LnPatchifyPG: x-adjacent tokens per warp iteration
+    const int pg = Cin <= 512 ? 4 : (Cin <= 1024 ? 2 : 1);  // LnPatchifyPG: x-adjacent tokens per warp iteration
     const long long groups = (long long)nb * H * ceil_div(W, pg);
     long long blocks = ceil_div<long long>(groups, 8);
     if (blocks > (long long)num_sms() * 8) blocks = (long long)num_sms() * 8;
@@ -1062,6 +1083,9 @@ static int launch_ln_patchify(const void* x, const DownParams& d, void* a2, int 
         case 192: ln_patchify_kernel<T, 192><<<(int)blocks, 256, 0, st>>>(xp, d.lnw, d.lnb, ap, nb, H, W); break;
         case 384: ln_patchify_kernel<T, 384><<<(int)blocks, 256, 0, st>>>(xp, d.lnw, d.lnb, ap, nb, H, W); break;
         case 768: ln_patchify_kernel<T, 768><<<(int)blocks, 256, 0, st>>>(xp, d.lnw, d.lnb, ap, nb, H, W); break;
+        case 352: ln_patchify_kernel<T, 352><<<(int)blocks, 256, 0, st>>>(xp, d.lnw, d.lnb, ap, nb, H, W); break;  // convnextv2_huge
+        case 704: ln_patchify_kernel<T, 704><<<(int)blocks, 256, 0, st>>>(xp, d.lnw, d.lnb, ap, nb, H, W); break;
+        case 1408: ln_patchify_kernel<T, 1408><<<(int)blocks, 256, 0, st>>>(xp, d.lnw, d.lnb, ap, nb, H, W); break;
         default: return set_error(SVB_ERR_UNSUPPORTED_MODEL, "ln_patchify: unsupported width %d", Cin);
     }
     SVB_LAUNCHED();
@@ -1087,8 +1111,10 @@ template <typename T>
 static int launch_head(const T* x, int nb, int tokens, int C, const float* n0w, const float* n0b, const float* n1w, const float* n1b,
                        const float* w1, const float* b1, int hid, const float* w2, const float* b2, int nout, float* coords,
                        cudaStream_t st) {
-    const size_t smem = (size_t)(C + hid + 8 + C + 8 * C) * 4;  // feat, hidden, reduction scratch, pool share, per-warp pools
-    SVB_REQUIRE(smem <= 99 * 1024, SVB_ERR_UNSUPPORTED_MODEL, "head: C=%d needs %zu bytes of shared memory", C, smem);
+    // feat, hidden, reduction scratch, pool share, per-warp pools: 81 KB at C = 2048, 111 KB at C = 2816 (convnextv2_huge: one CTA
+    // of the cluster per SM)
+    const size_t smem = (size_t)(C + hid + 8 + C + 8 * C) * 4;
+    SVB_REQUIRE(smem <= 227 * 1024, SVB_ERR_UNSUPPORTED_MODEL, "head: C=%d needs %zu bytes of shared memory", C, smem);
     auto kern = head_kernel<T>;
     static size_t attr_smem[MAX_DEVICES] = {};
     const int dslot = current_device_slot();
@@ -1176,14 +1202,18 @@ static int forward_chunk(svb_model* m, const uint8_t* in, const float* in_f32, i
         if (blocks > (long long)num_sms() * 4) blocks = (long long)num_sms() * 4;  // stem_ln_kernel: 4 resident CTAs per SM
         if (blocks < 1) blocks = 1;
         if (int rc = tm.begin(SVB_KC_STEM)) return rc;
-        if (in_f32 != nullptr)
+        if (in_f32 != nullptr && m->dims[0] <= 256)
             stem3_ln_kernel<T><<<(int)blocks, 256, 0, st>>>(in_f32, m->stem_w3, m->stem_b3, m->stem_lnw, m->stem_lnb, X, nb, H, W, m->dims[0]);
+        else if (in_f32 != nullptr)  // 352 channels (convnextv2_huge): 11 per lane
+            stem3_ln_kernel<T, 11><<<(int)blocks, 256, 0, st>>>(in_f32, m->stem_w3, m->stem_b3, m->stem_lnw, m->stem_lnb, X, nb, H, W, m->dims[0]);
         else if (m->dims[0] == 128)
             stem_ln_kernel<T, 4><<<(int)blocks, 256, 0, st>>>(in, m->stem_w, m->stem_b, m->stem_lnw, m->stem_lnb, X, nb, H, W);
         else if (m->dims[0] == 192)
             stem_ln_kernel<T, 6><<<(int)blocks, 256, 0, st>>>(in, m->stem_w, m->stem_b, m->stem_lnw, m->stem_lnb, X, nb, H, W);
         else if (m->dims[0] == 96)
             stem_ln_kernel<T, 4, 96><<<(int)blocks, 256, 0, st>>>(in, m->stem_w, m->stem_b, m->stem_lnw, m->stem_lnb, X, nb, H, W);
+        else if (m->dims[0] == 352)
+            stem_ln_kernel<T, 12, 352><<<(int)blocks, 256, 0, st>>>(in, m->stem_w, m->stem_b, m->stem_lnw, m->stem_lnb, X, nb, H, W);
         else
             stem_ln_kernel<T, 8><<<(int)blocks, 256, 0, st>>>(in, m->stem_w, m->stem_b, m->stem_lnw, m->stem_lnb, X, nb, H, W);
         SVB_LAUNCHED();
@@ -1349,7 +1379,7 @@ extern "C" int svb_model_forward_stages(svb_model* m, const uint8_t* d_in_u8, in
 extern "C" int svb_model_forward_f32(svb_model* m, const float* d_in_nchw, int B, int H, int W, float* d_coords,
                                      int micro_batch, void* d_ws, size_t ws_bytes, void* stream_, float* times_ms) {
     SVB_REQUIRE(d_in_nchw, SVB_ERR_INVALID_ARG, "model_forward_f32: null argument");
-    SVB_REQUIRE(!m || m->dims[0] <= 256, SVB_ERR_UNSUPPORTED_MODEL, "model_forward_f32: stem width %d > 256", m ? m->dims[0] : 0);
+    SVB_REQUIRE(!m || m->dims[0] <= 352, SVB_ERR_UNSUPPORTED_MODEL, "model_forward_f32: stem width %d > 352", m ? m->dims[0] : 0);
     return model_forward_any(m, nullptr, d_in_nchw, B, H, W, d_coords, micro_batch, d_ws, ws_bytes, stream_, times_ms);
 }
 
@@ -1447,6 +1477,7 @@ static int stem_entry(const uint8_t* in, const float* wf, const float* bf, const
     else if (C0 == 192) stem_ln_kernel<T, 6><<<(int)blocks, 256, 0, st>>>(in, wf, bf, lnw, lnb, static_cast<T*>(out), B, H, W);
     else if (C0 == 96) stem_ln_kernel<T, 4, 96><<<(int)blocks, 256, 0, st>>>(in, wf, bf, lnw, lnb, static_cast<T*>(out), B, H, W);
     else if (C0 == 256) stem_ln_kernel<T, 8><<<(int)blocks, 256, 0, st>>>(in, wf, bf, lnw, lnb, static_cast<T*>(out), B, H, W);
+    else if (C0 == 352) stem_ln_kernel<T, 12, 352><<<(int)blocks, 256, 0, st>>>(in, wf, bf, lnw, lnb, static_cast<T*>(out), B, H, W);
     else return set_error(SVB_ERR_UNSUPPORTED_MODEL, "stem: width %d unsupported", C0);
     SVB_LAUNCHED();
     return SVB_OK;

@@ -54,9 +54,13 @@ __global__ void __launch_bounds__(256, (CPL <= 4) ? 4 : 2) stem_ln_kernel(const 
                                                          int W) {
     static_assert(CPL % 2 == 0, "stem packs channel pairs");
     // C0 < 32 * CPL (96 channels with CPL = 4, convnext_tiny / small): the lanes past C0 / CPL carry zero weights, stay out of
-    // the LayerNorm sums and do not store
+    // the LayerNorm sums and do not store.  RAGGED (C0 % CPL != 0; 352 channels with CPL = 12, convnextv2_huge): one lane is
+    // only part-filled, so the same three things are done per channel pair (the off pairs of that lane are masked).  CPL = 12
+    // rather than 11 channels per lane because the FMAs work on packed pairs; 29 lanes of 12 + one of 4 keep the 2 CTAs per SM
+    // of the CPL = 8 (256-wide) stem.
     constexpr int NP = CPL / 2, TPW = STEM_TPW;
-    static_assert(C0 % CPL == 0 && C0 <= 32 * CPL, "stem width");
+    constexpr bool RAGGED = C0 % CPL != 0;
+    static_assert(C0 % 2 == 0 && C0 <= 32 * CPL, "stem width");
     // folded weights as packed channel pairs in shared memory, [tap][pair j][lane]: a warp's read of one (tap, j) is 256
     // contiguous bytes.  (In registers they cost 32 * NP registers per thread and held the kernel at 16 warps per SM, where
     // it is latency-bound; from shared memory each value is read once per TPW tokens.)
@@ -78,10 +82,19 @@ __global__ void __launch_bounds__(256, (CPL <= 4) ? 4 : 2) stem_ln_kernel(const 
 #pragma unroll
     for (int j = 0; j < NP; ++j) {
         const int c = lane * CPL + 2 * j;
-        bias2[j] = lane_on ? pk2(bf[c], bf[c + 1]) : pk2(0.f, 0.f);
+        if constexpr (RAGGED) bias2[j] = c < C0 ? pk2(bf[c], bf[c + 1]) : pk2(0.f, 0.f);
+        else bias2[j] = lane_on ? pk2(bf[c], bf[c + 1]) : pk2(0.f, 0.f);
     }
 #pragma unroll
-    for (int j = 0; j < CPL; ++j) { g[j] = lane_on ? lnw[lane * CPL + j] : 0.f; be[j] = lane_on ? lnb[lane * CPL + j] : 0.f; }
+    for (int j = 0; j < CPL; ++j) {
+        if constexpr (RAGGED) {
+            const int c = lane * CPL + j;
+            g[j] = c < C0 ? lnw[c] : 0.f;
+            be[j] = c < C0 ? lnb[c] : 0.f;
+        } else {
+            g[j] = lane_on ? lnw[lane * CPL + j] : 0.f; be[j] = lane_on ? lnb[lane * CPL + j] : 0.f;
+        }
+    }
     __syncthreads();
 
     const bool row_quad = (Wo % TPW) == 0;  // the TPW tokens of an iteration are x-adjacent: one 128-bit load per pixel row
@@ -152,6 +165,8 @@ __global__ void __launch_bounds__(256, (CPL <= 4) ? 4 : 2) stem_ln_kernel(const 
                 float lo, hi;
                 upk2(acc[k][j], lo, hi);
                 lo -= mean[k]; hi -= mean[k];
+                if constexpr (RAGGED)
+                    if (lane * CPL + 2 * j >= C0) continue;
                 q = fmaf(lo, lo, q);
                 q = fmaf(hi, hi, q);
             }
@@ -180,7 +195,11 @@ __global__ void __launch_bounds__(256, (CPL <= 4) ? 4 : 2) stem_ln_kernel(const 
             else if (NP == 4) *reinterpret_cast<uint4*>(op) = make_uint4(o[0], o[1], o[NP > 2 ? 2 : 0], o[NP > 3 ? 3 : 0]);
             else {
 #pragma unroll
-                for (int j = 0; j < NP; ++j) op[j] = o[j];
+                for (int j = 0; j < NP; ++j) {
+                    if constexpr (RAGGED)
+                        if (lane * CPL + 2 * j >= C0) continue;  // the part-filled lane: its pairs past C0
+                    op[j] = o[j];
+                }
             }
         }
     }
@@ -191,11 +210,11 @@ __global__ void __launch_bounds__(256, (CPL <= 4) ? 4 : 2) stem_ln_kernel(const 
 // hands to model(tensor) (generic.py:389-391).  Any caller that runs the module on its own tensor (notebooks,
 // BaseModel.test_inference) lands here; the dataset path uses the folded one-plane stem above.  One warp per token, lane =
 // C0 / 32 (rounded up) consecutive channels; the 48 inputs of the patch are read once per token and broadcast.
-template <typename T>
+// MAXC: channels per lane, C0 <= 32 * MAXC (8 up to 256 channels, 11 for convnextv2_huge's 352).
+template <typename T, int MAXC = 8>
 __global__ void __launch_bounds__(256) stem3_ln_kernel(const float* __restrict__ in, const float* __restrict__ w /*[C0][48] = [co][ci][ky][kx]*/,
                                                       const float* __restrict__ bias, const float* __restrict__ lnw,
                                                       const float* __restrict__ lnb, T* __restrict__ out, int B, int H, int W, int C0) {
-    constexpr int MAXC = 8;  // channels per lane: C0 <= 256
     const int lane = threadIdx.x & 31;
     const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
@@ -546,7 +565,8 @@ dwconv_ln_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_constan
 //   * the A operand is not rounded a second time after normalisation: predicted AND measured coordinate error goes DOWN
 //     (scripts/emulate_precision.py: fp16 trained-like 0.176 -> 0.119 px)
 // The statistics are taken from the fp32 results before rounding (mean of the rounded values differs by the MEAN rounding error,
-// 2^-12 |y| / sqrt(C): far below one element's rounding).  One pass: var = E[y^2] - mu^2 in fp32 over C <= 2048 values.
+// 2^-12 |y| / sqrt(C): far below one element's rounding).  One pass: var = E[y^2] - mu^2 in fp32 over C <= 2816 values
+// (convnextv2_huge's last stage; each lane adds C / 64 values per pixel, the 32 lane sums meet in a shuffle tree).
 // Per thread 16 pixels x packed (sum, sum of squares) pairs have to live across the channel chunks; 64 more registers next to
 // the convolution's 88 would spill, so between chunks they are parked in TENSOR MEMORY (two tcgen05.st / .ld pairs per chunk,
 // against 784 FFMA2) -- the epilogue of a chunk is then one F2FP, one STG and two packed FMA-pipe operations per pixel.
@@ -2228,7 +2248,8 @@ __global__ void __launch_bounds__(256) grn_apply_kernel(T* __restrict__ h, int t
 // ============================================================================ LayerNorm2d + 2x2/s2 patchify
 // x [B,H,W,C] -> a2 [B,H/2,W/2,4C] with k = (ky*2+kx)*C + c, the A operand of the downsample GEMM
 // (timm stage.downsample = LayerNorm2d -> Conv2d(k=2,s=2)).
-template <int C> struct LnPatchifyPG { static constexpr int value = C <= 512 ? 4 : 2; };
+// 1408 channels (convnextv2_huge stage 2, V4 = 11) at PG = 2 need 160 registers, one CTA per SM: one token per iteration keeps two
+template <int C> struct LnPatchifyPG { static constexpr int value = C <= 512 ? 4 : (C <= 1024 ? 2 : 1); };
 
 template <typename T, int C>
 __global__ void __launch_bounds__(256) ln_patchify_kernel(const T* __restrict__ x, const float* __restrict__ lnw,
@@ -2237,8 +2258,8 @@ __global__ void __launch_bounds__(256) ln_patchify_kernel(const T* __restrict__ 
     // One warp = PG x-adjacent tokens per iteration: PG independent load / reduction chains in flight, the index arithmetic
     // (three divisions) paid once per PG tokens, and the two LayerNorm reductions of all PG tokens in one recursive-halving
     // pass (warp_sum4).  A lane owns 4 consecutive channels of every 128-channel group.
-    constexpr int V4 = (C + 127) / 128;  // a lane's 4-channel groups; the last one is half empty when C % 128 == 64 (192-wide)
-    constexpr int PG = LnPatchifyPG<C>::value;  // 4, or 2 beyond 512 channels (registers)
+    constexpr int V4 = (C + 127) / 128;  // a lane's 4-channel groups; the last one is part empty when C % 128 != 0 (192, 352, 704)
+    constexpr int PG = LnPatchifyPG<C>::value;  // 4, 2 beyond 512 channels, 1 beyond 1024 (registers)
     const int lane = threadIdx.x & 31;
     const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;

@@ -27,7 +27,7 @@ from typing import Literal
 
 import numpy as np
 import torch
-from pydantic import field_validator, BaseModel, ConfigDict, computed_field
+from pydantic import BaseModel, ConfigDict, computed_field
 
 from . import hostio, ops, pipeline, volumes
 from .cropping import LocalizationModel, load_localization_model
@@ -67,17 +67,6 @@ class ClassificationDatasetConfig(BaseModel):
     chunk_series: int = 128
     io_threads: int = 0
     png_level: int = 6
-
-    @field_validator("model_variant")
-    @classmethod
-    def _variant_is_built(cls, v: str) -> str:
-        # the reference's Literal lists v2_huge (config.py:27-39); this build's depthwise kernel stops at 2048 channels
-        # (convnextv2_huge: 352 / 704 / 1408 / 2816), so the configuration is refused when it is MADE, not after the
-        # label files have been read and the checkpoint loaded
-        if v == "v2_huge":
-            raise ValueError("model_variant='v2_huge' (convnextv2_huge, 2816 channels) is not built in spine_vision_b200: "
-                             "supported variants are tiny, small, base, large, xlarge, v2_tiny, v2_small, v2_base, v2_large")
-        return v
 
     @computed_field
     @property
