@@ -11,10 +11,11 @@
  * Conventions
  *  - every pointer named d_* is a DEVICE pointer owned by the caller
  *    (PyTorch tensors: tensor.data_ptr()); workspaces are caller-owned too.
- *    The library owns only svb_model handles.
+ *    The library owns only svb_model and svb_model_graph handles.
  *  - calls are asynchronous on `stream` (a cudaStream_t passed as void*),
  *    with no hidden synchronisation or allocation, except svb_model_create /
- *    svb_model_destroy which allocate and synchronise.
+ *    svb_model_destroy which allocate and synchronise, and
+ *    svb_model_graph_create which allocates.
  *  - return value: 0 on success, negative svb_status otherwise; the message
  *    is available from svb_last_error() (thread local).  Nothing throws.
  *  - there is no CPU fallback: a device that is not sm_100 gives
@@ -236,6 +237,30 @@ int svb_model_forward_f32(svb_model* m, const float* d_in_nchw, int B, int H, in
  * of the model dtype, written by one device-to-device copy per micro-batch on the stream that computed it.  1 <= n_stage_out <= 4. */
 int svb_model_forward_stages(svb_model* m, const uint8_t* d_in_u8, int B, int H, int W, float* d_coords, int micro_batch,
                              void* d_ws, size_t ws_bytes, void* stream, void* const* d_stage_out, int n_stage_out);
+/* CUDA graph of one svb_model_forward / svb_model_forward_f32: the same kernels, micro-batches, second chain, tail micro-batch,
+ * programmatic dependent launches and clusters, captured once and replayed with one cudaGraphLaunch per call.
+ *  create  : checks its arguments as svb_model_forward does, captures one forward over B images of H x W with `micro_batch` on
+ *            `stream` (thread-local capture mode; not the legacy default stream, and not a stream that is already capturing)
+ *            and instantiates it (allocating what the graph needs; nothing is enqueued on `stream`).  A capture that fails is ended and discarded: the call returns a negative svb_status and the
+ *            stream stays usable.  input_kind: SVB_GRAPH_INPUT_U8 (uint8 [B,H,W] planes, folded stem) or SVB_GRAPH_INPUT_F32
+ *            (float32 [B,3,H,W], as svb_model_forward_f32).
+ *  launch  : d_in / d_coords may differ on every call (the nodes that read the input and write the coordinates are rebound; a
+ *            replay already enqueued keeps its pointers).  Asynchronous on `stream`; adds the graph's kernel-node count to
+ *            svb_launch_count.  Replays of one graph run one after another, whatever stream they are launched on.
+ *  info    : out[0] = kernel nodes (the launches of one svb_model_forward with the same arguments), out[1..3] = B, H, W.
+ * The graph binds d_ws for its lifetime and owns no workspace: the caller keeps it alive and does not use it for anything else
+ * while the graph exists.  Destroy the graph before its model.  Shapes are fixed at capture: another B, H, W or micro-batch is
+ * another graph.  Per-stage readout (svb_model_forward_stages) and per-launch timing (times_ms) are not supported in graphs; a
+ * svb_model_forward / svb_model_forward_f32 on a stream that is capturing records correctly (torch.cuda.graph), but refuses
+ * times_ms with SVB_ERR_INVALID_ARG.  A handle is not thread-safe, like svb_model. */
+typedef struct svb_model_graph svb_model_graph;
+#define SVB_GRAPH_INPUT_U8 0  /* svb_model_forward: uint8 [B,H,W] planes, folded stem */
+#define SVB_GRAPH_INPUT_F32 1 /* svb_model_forward_f32: float32 [B,3,H,W], model(tensor) */
+int svb_model_graph_create(svb_model* m, int input_kind, int B, int H, int W, int micro_batch, void* d_ws, size_t ws_bytes,
+                           void* stream, svb_model_graph** out);
+int svb_model_graph_launch(svb_model_graph* g, const void* d_in, float* d_coords, void* stream);
+int svb_model_graph_info(const svb_model_graph* g, int32_t out[4]); /* kernel nodes, B, H, W */
+int svb_model_graph_destroy(svb_model_graph* g);
 /* model geometry: out[0]=num_levels, out[1]=num_outputs, out[2..5]=dims, out[6..9]=depths */
 int svb_model_info(const svb_model* m, int32_t out[10]);
 /* total tensor-core GEMM flops and launches of one forward over B images (for the roofline) */

@@ -16,6 +16,7 @@ LIB_PATH = Path(os.environ.get("SPINE_B200_LIB", _PKG / "libspine_b200.so"))
 SVB_BF16, SVB_FP16, SVB_F32 = 0, 1, 2
 PIXEL_FLOAT, PIXEL_INT16, PIXEL_UINT16, PIXEL_UINT8 = 0, 1, 2, 3  # SVB_PIXEL_*: the file's pixel type of a slice (rotated crops)
 DTYPES = {"bf16": SVB_BF16, "bfloat16": SVB_BF16, "fp16": SVB_FP16, "float16": SVB_FP16, "half": SVB_FP16}
+GRAPH_INPUT_U8, GRAPH_INPUT_F32 = 0, 1  # SVB_GRAPH_INPUT_*: what a captured forward reads
 KERNEL_CLASSES = ("stem", "dwconv_ln", "gemm", "ln_patchify", "head", "mlp_fused")
 
 # every symbol include/spine_b200.h declares
@@ -26,7 +27,7 @@ EXPORTS = (
     "svb_k1_workspace_bytes", "svb_k1_normalize_resize", "svb_normalize_u8_workspace_bytes", "svb_normalize_u8",
     "svb_k3_workspace_bytes", "svb_k3_crop_resample", "svb_k3_crop_resample_rotated",
     "svb_model_create", "svb_model_destroy", "svb_model_workspace_bytes", "svb_model_forward", "svb_model_forward_f32",
-    "svb_model_forward_stages",
+    "svb_model_forward_stages", "svb_model_graph_create", "svb_model_graph_launch", "svb_model_graph_info", "svb_model_graph_destroy",
     "svb_model_info", "svb_model_cost", "svb_gemm", "svb_mlp_fused", "svb_mlp_fused_ln",
     "svb_stem_ln", "svb_dwconv_ln", "svb_dwconv_raw", "svb_dwconv_tc_pack", "svb_dwconv_raw_tc", "svb_dwconv_ln_tc", "svb_ln_patchify", "svb_head",
     "svb_k4_classifier_input",
@@ -117,6 +118,14 @@ def load() -> C.CDLL:
     lib.svb_model_forward_f32.argtypes = [vp, vp, i32, i32, i32, vp, i32, vp, sz, vp, vp]
     lib.svb_model_forward_stages.restype = C.c_int
     lib.svb_model_forward_stages.argtypes = [vp, vp, i32, i32, i32, vp, i32, vp, sz, vp, C.POINTER(vp), i32]
+    lib.svb_model_graph_create.restype = C.c_int
+    lib.svb_model_graph_create.argtypes = [vp, i32, i32, i32, i32, i32, vp, sz, vp, C.POINTER(vp)]
+    lib.svb_model_graph_launch.restype = C.c_int
+    lib.svb_model_graph_launch.argtypes = [vp, vp, vp, vp]
+    lib.svb_model_graph_info.restype = C.c_int
+    lib.svb_model_graph_info.argtypes = [vp, C.POINTER(C.c_int32 * 4)]
+    lib.svb_model_graph_destroy.restype = C.c_int
+    lib.svb_model_graph_destroy.argtypes = [vp]
     lib.svb_model_info.restype = C.c_int
     lib.svb_model_info.argtypes = [vp, C.POINTER(C.c_int32 * 10)]
     lib.svb_model_cost.restype = C.c_int

@@ -23,7 +23,7 @@ int set_error(int code, const char* fmt, ...) {
 }
 
 static std::atomic<long long> g_launches{0};
-void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
+void count_launch(long long n) { g_launches.fetch_add(n, std::memory_order_relaxed); }
 long long launches_total(bool reset) { return reset ? g_launches.exchange(0) : g_launches.load(); }
 
 int check_device_sm100() {

@@ -32,8 +32,8 @@ int set_error(int code, const char* fmt, ...);
         if (!(cond)) return svb::set_error((code), __VA_ARGS__);                                   \
     } while (0)
 
-// every kernel launch of the library is counted (bench.py reports it as gpu_launches)
-void count_launch();
+// every kernel launch of the library is counted (bench.py reports it as gpu_launches); a CUDA graph replay adds its kernel nodes
+void count_launch(long long n = 1);
 #define SVB_LAUNCHED()                          \
     do {                                        \
         svb::count_launch();                    \

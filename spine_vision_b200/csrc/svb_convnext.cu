@@ -1317,11 +1317,10 @@ extern "C" size_t svb_model_workspace_bytes(const svb_model* m, int micro_batch,
     return dual_chain_enabled() ? 2 * one : one;
 }
 
-static int model_forward_any(svb_model* m, const uint8_t* d_in_u8, const float* d_in_f32, int B, int H, int W, float* d_coords,
-                             int micro_batch, void* d_ws, size_t ws_bytes, void* stream_, float* times_ms,
-                             void* const* stage_out = nullptr, int n_stage_out = 0) {
-    cudaStream_t st = static_cast<cudaStream_t>(stream_);
-    SVB_REQUIRE(m && (d_in_u8 || d_in_f32) && d_coords && d_ws, SVB_ERR_INVALID_ARG, "model_forward: null argument");
+// the argument checks of model_forward_any, also made by svb_model_graph_create before it begins a capture
+static int check_forward_args(const svb_model* m, const void* d_in, const float* d_coords, int B, int H, int W, int micro_batch,
+                              const void* d_ws, size_t ws_bytes) {
+    SVB_REQUIRE(m && d_in && d_coords && d_ws, SVB_ERR_INVALID_ARG, "model_forward: null argument");
     SVB_REQUIRE(B >= 0 && micro_batch > 0, SVB_ERR_INVALID_ARG, "model_forward: B=%d micro_batch=%d", B, micro_batch);
     SVB_REQUIRE(H > 0 && W > 0 && H % 32 == 0 && W % 32 == 0, SVB_ERR_INVALID_ARG,
                 "model_forward: input %dx%d must be a positive multiple of 32 (ConvNeXt stride)", H, W);
@@ -1329,6 +1328,22 @@ static int model_forward_any(svb_model* m, const uint8_t* d_in_u8, const float* 
     const size_t need = ws_layout(m, micro_batch, H, W).total;
     SVB_REQUIRE(ws_bytes >= need, SVB_ERR_WORKSPACE_TOO_SMALL, "model_forward: workspace %zu < %zu bytes", ws_bytes, need);
     SVB_REQUIRE((reinterpret_cast<uintptr_t>(d_ws) & 1023) == 0, SVB_ERR_INVALID_ARG, "model_forward: workspace must be 1024-byte aligned");
+    return SVB_OK;
+}
+
+static int model_forward_any(svb_model* m, const uint8_t* d_in_u8, const float* d_in_f32, int B, int H, int W, float* d_coords,
+                             int micro_batch, void* d_ws, size_t ws_bytes, void* stream_, float* times_ms,
+                             void* const* stage_out = nullptr, int n_stage_out = 0) {
+    cudaStream_t st = static_cast<cudaStream_t>(stream_);
+    const void* d_in = d_in_u8 ? static_cast<const void*>(d_in_u8) : static_cast<const void*>(d_in_f32);
+    if (int rc = check_forward_args(m, d_in, d_coords, B, H, W, micro_batch, d_ws, ws_bytes)) return rc;
+    if (times_ms) {  // Timer::finish synchronises, which a stream capture (CUDA graph) does not allow
+        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+        SVB_CUDA_OK(cudaStreamIsCapturing(st, &cap));
+        SVB_REQUIRE(cap == cudaStreamCaptureStatusNone, SVB_ERR_INVALID_ARG, "model_forward: times_ms is not supported while the stream is capturing");
+    }
+    if (micro_batch > B && B > 0) micro_batch = B;
+    const size_t need = ws_layout(m, micro_batch, H, W).total;
     Timer tm{m, st, times_ms != nullptr};
     const size_t one = align_up(need, 1024);
     const bool dual = dual_chain_enabled() && times_ms == nullptr && B > micro_batch && ws_bytes >= 2 * one && m->aux_stream != nullptr;
@@ -1352,7 +1367,13 @@ static int model_forward_any(svb_model* m, const uint8_t* d_in_u8, const float* 
             rc = forward_chunk<__half>(m, in8, in32, nb, H, W, d_coords + (size_t)b0 * m->nout, ws, cs, tm, so, n_stage_out);
         else
             rc = forward_chunk<__nv_bfloat16>(m, in8, in32, nb, H, W, d_coords + (size_t)b0 * m->nout, ws, cs, tm, so, n_stage_out);
-        if (rc) return rc;
+        if (rc) {
+            if (dual) {  // join anyway: a capture that fails here must not leave the handle's stream part of it
+                cudaEventRecord(m->join_ev, m->aux_stream);
+                cudaStreamWaitEvent(st, m->join_ev, 0);
+            }
+            return rc;
+        }
     }
     if (dual) {
         SVB_CUDA_OK(cudaEventRecord(m->join_ev, m->aux_stream));
@@ -1381,6 +1402,146 @@ extern "C" int svb_model_forward_f32(svb_model* m, const float* d_in_nchw, int B
     SVB_REQUIRE(d_in_nchw, SVB_ERR_INVALID_ARG, "model_forward_f32: null argument");
     SVB_REQUIRE(!m || m->dims[0] <= 352, SVB_ERR_UNSUPPORTED_MODEL, "model_forward_f32: stem width %d > 352", m ? m->dims[0] : 0);
     return model_forward_any(m, nullptr, d_in_nchw, B, H, W, d_coords, micro_batch, d_ws, ws_bytes, stream_, times_ms);
+}
+
+// ---- CUDA graph of one forward ----------------------------------------------------------------
+struct svb_model_graph {
+    struct Bind {  // a kernel node with an argument that addresses the caller's input or coordinates
+        cudaGraphNode_t node;
+        cudaKernelNodeParams params;  // as captured; the argument values belong to the node (alive while `graph` is)
+        std::vector<void*> args;      // pointers to the node's argument values, args[arg] replaced at launch
+        int arg;
+        bool coords;                  // the argument addresses the coordinates (else the input)
+        uintptr_t offset;             // bytes from the caller's base pointer: the micro-batch's first image
+        uintptr_t value;
+    };
+    int B = 0, H = 0, W = 0;
+    long long kernel_nodes = 0;
+    cudaGraph_t graph = nullptr;
+    cudaGraphExec_t exec = nullptr;
+    std::vector<Bind> binds;
+    const void* bound_in = nullptr;  // what the nodes were last rebound to
+    const float* bound_coords = nullptr;
+    ~svb_model_graph() {
+        if (exec) cudaGraphExecDestroy(exec);
+        if (graph) cudaGraphDestroy(graph);
+    }
+};
+
+// The capture runs with placeholder addresses for the caller's input and coordinates, far outside any allocation (the kernels
+// of a capture do not run); every kernel argument that falls in one of the two ranges marks a node to rebind at launch.
+static constexpr uintptr_t GRAPH_IN_BASE = 0x7e10000000000000ull, GRAPH_COORDS_BASE = 0x7e20000000000000ull;
+
+static int graph_find_binds(svb_model_graph* g, size_t in_bytes, size_t coords_bytes) {
+    size_t n = 0;
+    SVB_CUDA_OK(cudaGraphGetNodes(g->graph, nullptr, &n));
+    std::vector<cudaGraphNode_t> nodes(n);
+    SVB_CUDA_OK(cudaGraphGetNodes(g->graph, nodes.data(), &n));
+    for (cudaGraphNode_t node : nodes) {
+        cudaGraphNodeType type;
+        SVB_CUDA_OK(cudaGraphNodeGetType(node, &type));
+        if (type != cudaGraphNodeTypeKernel) continue;
+        ++g->kernel_nodes;
+        cudaKernelNodeParams p;
+        SVB_CUDA_OK(cudaGraphKernelNodeGetParams(node, &p));
+        SVB_REQUIRE(p.kernelParams != nullptr, SVB_ERR_CUDA, "model_graph_create: a kernel node without an argument array");
+        size_t nargs = 0, off = 0, size = 0;
+        while (cudaFuncGetParamInfo(p.func, nargs, &off, &size) == cudaSuccess) ++nargs;
+        cudaGetLastError();  // the query past the last argument fails by design; do not leave that for the next launch check
+        for (size_t i = 0; i < nargs; ++i) {
+            SVB_CUDA_OK(cudaFuncGetParamInfo(p.func, i, &off, &size));
+            if (size != sizeof(uintptr_t)) continue;
+            uintptr_t v;
+            memcpy(&v, p.kernelParams[i], sizeof(v));
+            const bool in = v - GRAPH_IN_BASE < in_bytes, out = v - GRAPH_COORDS_BASE < coords_bytes;
+            if (!in && !out) continue;
+            svb_model_graph::Bind b{node, p, std::vector<void*>(p.kernelParams, p.kernelParams + nargs), (int)i, out,
+                                    v - (out ? GRAPH_COORDS_BASE : GRAPH_IN_BASE), 0};
+            g->binds.push_back(std::move(b));
+        }
+    }
+    return SVB_OK;
+}
+
+extern "C" int svb_model_graph_create(svb_model* m, int input_kind, int B, int H, int W, int micro_batch, void* d_ws, size_t ws_bytes,
+                                      void* stream_, svb_model_graph** out) {
+    SVB_REQUIRE(out, SVB_ERR_INVALID_ARG, "model_graph_create: null argument");
+    *out = nullptr;
+    SVB_REQUIRE(input_kind == SVB_GRAPH_INPUT_U8 || input_kind == SVB_GRAPH_INPUT_F32, SVB_ERR_INVALID_ARG,
+                "model_graph_create: input_kind %d", input_kind);
+    SVB_REQUIRE(B > 0, SVB_ERR_INVALID_ARG, "model_graph_create: B=%d (a graph holds at least one image)", B);
+    const bool f32 = input_kind == SVB_GRAPH_INPUT_F32;
+    const void* in = reinterpret_cast<const void*>(GRAPH_IN_BASE);
+    float* coords = reinterpret_cast<float*>(GRAPH_COORDS_BASE);
+    if (int rc = check_forward_args(m, in, coords, B, H, W, micro_batch, d_ws, ws_bytes)) return rc;
+    SVB_REQUIRE(!f32 || m->dims[0] <= 352, SVB_ERR_UNSUPPORTED_MODEL, "model_forward_f32: stem width %d > 352", m->dims[0]);
+    cudaStream_t st = static_cast<cudaStream_t>(stream_);
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    SVB_CUDA_OK(cudaStreamIsCapturing(st, &cap));
+    SVB_REQUIRE(cap == cudaStreamCaptureStatusNone, SVB_ERR_INVALID_ARG, "model_graph_create: the stream is already capturing");
+
+    std::unique_ptr<svb_model_graph> g(new svb_model_graph());
+    g->B = B;
+    g->H = H;
+    g->W = W;
+    const cudaError_t begin = cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal);
+    if (begin != cudaSuccess) {  // e.g. the legacy default stream; not sticky: keep it from failing the next launch check
+        cudaGetLastError();
+        return set_error(SVB_ERR_CUDA, "model_graph_create: cannot capture on this stream: %s", cudaGetErrorString(begin));
+    }
+    int rc = model_forward_any(m, f32 ? nullptr : static_cast<const uint8_t*>(in), f32 ? static_cast<const float*>(in) : nullptr, B, H, W,
+                               coords, micro_batch, d_ws, ws_bytes, st, nullptr);
+    const cudaError_t end = cudaStreamEndCapture(st, &g->graph);  // ends the capture whatever happened in it
+    if (end != cudaSuccess) cudaGetLastError();  // not sticky: keep it from failing the next launch check
+    if (rc) return rc;
+    SVB_REQUIRE(end == cudaSuccess && g->graph != nullptr, SVB_ERR_CUDA, "model_graph_create: the capture failed: %s", cudaGetErrorString(end));
+    const size_t in_bytes = (size_t)B * H * W * (f32 ? 3 * sizeof(float) : 1), coords_bytes = (size_t)B * m->nout * sizeof(float);
+    if (int rc2 = graph_find_binds(g.get(), in_bytes, coords_bytes)) return rc2;
+    count_launch(-g->kernel_nodes);  // the capture counted one launch per kernel node, and none of them ran
+    // every micro-batch has one stem that reads the input and one head that writes the coordinates, and nothing else touches either
+    const int mb = micro_batch < B ? micro_batch : B;
+    const long long chunks = (B + mb - 1) / mb;
+    long long n_in = 0, n_coords = 0;
+    for (const auto& b : g->binds) (b.coords ? n_coords : n_in) += 1;
+    SVB_REQUIRE(n_in == chunks && n_coords == chunks, SVB_ERR_CUDA,
+                "model_graph_create: %lld input and %lld coordinate arguments in the graph, expected %lld of each", n_in, n_coords, chunks);
+    SVB_CUDA_OK(cudaGraphInstantiate(&g->exec, g->graph, 0));
+    *out = g.release();
+    return SVB_OK;
+}
+
+extern "C" int svb_model_graph_launch(svb_model_graph* g, const void* d_in, float* d_coords, void* stream_) {
+    SVB_REQUIRE(g && d_in && d_coords, SVB_ERR_INVALID_ARG, "model_graph_launch: null argument");
+    if (d_in != g->bound_in || d_coords != g->bound_coords) {
+        // changes only launches enqueued from here on: a replay still in flight keeps the pointers it was launched with
+        for (auto& b : g->binds) {
+            b.value = reinterpret_cast<uintptr_t>(b.coords ? static_cast<const void*>(d_coords) : d_in) + b.offset;
+            b.args[b.arg] = &b.value;
+            cudaKernelNodeParams p = b.params;
+            p.kernelParams = b.args.data();
+            p.extra = nullptr;
+            SVB_CUDA_OK(cudaGraphExecKernelNodeSetParams(g->exec, b.node, &p));
+        }
+        g->bound_in = d_in;
+        g->bound_coords = d_coords;
+    }
+    SVB_CUDA_OK(cudaGraphLaunch(g->exec, static_cast<cudaStream_t>(stream_)));
+    count_launch(g->kernel_nodes);
+    return SVB_OK;
+}
+
+extern "C" int svb_model_graph_info(const svb_model_graph* g, int32_t out[4]) {
+    SVB_REQUIRE(g && out, SVB_ERR_INVALID_ARG, "model_graph_info: null argument");
+    out[0] = (int32_t)g->kernel_nodes;
+    out[1] = g->B;
+    out[2] = g->H;
+    out[3] = g->W;
+    return SVB_OK;
+}
+
+extern "C" int svb_model_graph_destroy(svb_model_graph* g) {
+    delete g;
+    return SVB_OK;
 }
 
 extern "C" int svb_model_cost(const svb_model* m, int B, int H, int W, double* gemm_flops, int64_t* launches) {

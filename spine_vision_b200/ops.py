@@ -387,7 +387,7 @@ class LocalizationEngine:
             return coords
         mb = min(self.micro_batch, B)
         need = lib.svb_model_workspace_bytes(self._h, mb, H, W)
-        ws = _Workspace.get("model", need, u8.device)
+        ws = self._workspace(need, u8.device)
         wp, wn = _aligned_ptr(ws, 1024)
         if stage_out is not None:
             assert times is None, "per-stage readout is not timed"
@@ -420,11 +420,83 @@ class LocalizationEngine:
         mb = min(self.micro_batch, B)
         with torch.cuda.device(x.device):
             need = lib.svb_model_workspace_bytes(self._h, mb, H, W)
-            ws = _Workspace.get("model", need, x.device)
+            ws = self._workspace(need, x.device)
             wp, wn = _aligned_ptr(ws, 1024)
             _lib.check(lib.svb_model_forward_f32(self._h, x.data_ptr(), B, H, W, coords.data_ptr(), mb, wp, wn,
                                                  torch.cuda.current_stream(x.device).cuda_stream, None))
         return coords
+
+    @staticmethod
+    def _workspace(need: int, device) -> torch.Tensor:
+        if torch.cuda.is_current_stream_capturing():
+            # torch.cuda.graph: a workspace of this capture's own, from the graph's private memory pool, which keeps it for the
+            # graph's replays.  The shared one may be reallocated by a later, larger eager call while the graph still uses it.
+            return torch.empty(need + 1024, dtype=torch.uint8, device=device)
+        return _Workspace.get("model", need, device)
+
+    def capture(self, B: int, H: int, W: int, f32: bool = False) -> "GraphedForward":
+        """Capture one forward over ``B`` images of ``H`` x ``W`` as a CUDA graph (``svb_model_graph_create``): the same kernels
+        and schedule as ``forward`` (``f32=False``, uint8 ``[B,H,W]`` planes) or ``forward_tensor`` (``f32=True``, float32
+        ``[B,3,H,W]``), replayed by one ``cudaGraphLaunch`` per call.  The graph gets a workspace of its own, as large as the one
+        ``forward`` uses (about 3.3 GB for ``base`` at 512^2 with micro-batch 64 and two chains), held until the returned object
+        is released.  Shapes are fixed: another shape is another capture."""
+        return GraphedForward(self, int(B), int(H), int(W), bool(f32))
+
+
+class GraphedForward:
+    """A ``LocalizationEngine`` forward captured as a CUDA graph (``LocalizationEngine.capture``).  Calling it with a new input
+    replays the graph on the current stream; the input and the output may be different tensors on every call (nothing is
+    copied).  It keeps its engine, and so the model, alive, and owns a model workspace (one more ``forward`` workspace of
+    device memory).  Like the engine it is not thread-safe."""
+
+    def __init__(self, engine: LocalizationEngine, B: int, H: int, W: int, f32: bool):
+        index = engine.device.index if engine.device.index is not None else torch.cuda.current_device()
+        self.engine, self.device, self.f32 = engine, torch.device("cuda", index), f32
+        self.shape = (B, 3, H, W) if f32 else (B, H, W)
+        self.dtype = torch.float32 if f32 else torch.uint8
+        self.out_shape = (B, engine.num_levels, engine.num_outputs)
+        lib = _lib.load()
+        mb = min(engine.micro_batch, B)
+        with torch.cuda.device(self.device):
+            need = lib.svb_model_workspace_bytes(engine._h, mb, H, W)
+            self._ws = torch.empty(need + 1024, dtype=torch.uint8, device=self.device)
+            self._ws_stream = torch.cuda.current_stream(self.device)
+            wp, wn = _aligned_ptr(self._ws, 1024)
+            side = torch.cuda.Stream(self.device)  # the capture cannot begin on the legacy default stream
+            handle = C.c_void_p()
+            _lib.check(lib.svb_model_graph_create(engine._h, _lib.GRAPH_INPUT_F32 if f32 else _lib.GRAPH_INPUT_U8, B, H, W, mb, wp, wn,
+                                                  side.cuda_stream, C.byref(handle)))
+        self._h = handle
+        info = (C.c_int32 * 4)()
+        _lib.check(lib.svb_model_graph_info(self._h, C.byref(info)))
+        self.kernel_nodes = int(info[0])
+
+    def __del__(self):
+        h, self._h = getattr(self, "_h", None), None
+        if h:
+            try:
+                _lib.load().svb_model_graph_destroy(h)
+            except Exception:
+                pass
+
+    @_on_device
+    def __call__(self, x: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:
+        """Replay on ``x`` (the captured shape and dtype, contiguous, on the engine's device) -> float32
+        ``[B, num_levels, 2]``, written into ``out`` if given."""
+        if not isinstance(x, torch.Tensor) or tuple(x.shape) != self.shape or x.dtype != self.dtype:
+            got = (tuple(x.shape), x.dtype) if isinstance(x, torch.Tensor) else type(x).__name__
+            raise ValueError(f"graph captured for {self.dtype} {self.shape}, got {got}")
+        if x.device != self.device or not x.is_contiguous():
+            raise ValueError(f"graph input must be contiguous on {self.device}, got {x.device} (contiguous: {x.is_contiguous()})")
+        if out is None:
+            out = torch.empty(self.out_shape, dtype=torch.float32, device=self.device)
+        elif tuple(out.shape) != self.out_shape or out.dtype != torch.float32 or out.device != self.device or not out.is_contiguous():
+            raise ValueError(f"out must be a contiguous float32 {self.out_shape} tensor on {self.device}")
+        st = torch.cuda.current_stream(self.device)
+        if st != self._ws_stream:  # the workspace must not be handed out again while a replay on another stream may use it
+            self._ws.record_stream(st)
+        _lib.check(_lib.load().svb_model_graph_launch(self._h, x.data_ptr(), out.data_ptr(), st.cuda_stream))
+        return out
 
 
 @_on_device
