@@ -314,10 +314,6 @@ int svb_dwconv_tc_pack(const float* h_taps, void* h_wtc, int C, int dtype);
 int svb_dwconv_raw_tc(const void* d_x, const void* d_wtc, const float* d_bias, void* d_out, float* d_rowstat, float* d_stat_part, int B,
                       int H, int W, int C, int dtype, void* stream);
 
-/* The first tensor-core version (one MMA per tap; measured slower, kept as evidence): shifted-view diagonal tcgen05 MMAs; taps16 = the taps as 16-bit
- * [49][C] of `dtype`.  Supported for C = 256 / 512 while the halo tile fits in shared memory, else SVB_ERR_UNSUPPORTED_MODEL. */
-int svb_dwconv_ln_tc(const void* d_x, const void* d_taps16, const float* d_bias, const float* d_lnw,
-                     const float* d_lnb, void* d_out, int B, int H, int W, int C, int dtype, void* stream);
 int svb_ln_patchify(const void* d_x, const float* d_lnw, const float* d_lnb, void* d_out, int B, int H, int W,
                     int C, int dtype, void* stream);
 int svb_head(const void* d_x, int B, int tokens, int C, const float* n0w, const float* n0b, const float* n1w,

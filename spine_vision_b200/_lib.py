@@ -29,7 +29,7 @@ EXPORTS = (
     "svb_model_create", "svb_model_destroy", "svb_model_workspace_bytes", "svb_model_forward", "svb_model_forward_f32",
     "svb_model_forward_stages", "svb_model_graph_create", "svb_model_graph_launch", "svb_model_graph_info", "svb_model_graph_destroy",
     "svb_model_info", "svb_model_cost", "svb_gemm", "svb_mlp_fused", "svb_mlp_fused_ln",
-    "svb_stem_ln", "svb_dwconv_ln", "svb_dwconv_raw", "svb_dwconv_tc_pack", "svb_dwconv_raw_tc", "svb_dwconv_ln_tc", "svb_ln_patchify", "svb_head",
+    "svb_stem_ln", "svb_dwconv_ln", "svb_dwconv_raw", "svb_dwconv_tc_pack", "svb_dwconv_raw_tc", "svb_ln_patchify", "svb_head",
     "svb_k4_classifier_input",
     "svb_png_bound", "svb_png_encode_gray8", "svb_png_write_gray8_batch", "svb_png_write_gray8_ragged",
     "svb_mha_read_header", "svb_mha_read_f32", "svb_mha_read_batch_f32", "svb_mha_read_batch_slab_f32",
@@ -146,8 +146,6 @@ def load() -> C.CDLL:
     lib.svb_dwconv_tc_pack.argtypes = [vp, vp, i32, i32]
     lib.svb_dwconv_raw_tc.restype = C.c_int
     lib.svb_dwconv_raw_tc.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, vp]
-    lib.svb_dwconv_ln_tc.restype = C.c_int
-    lib.svb_dwconv_ln_tc.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, vp]
     lib.svb_ln_patchify.restype = C.c_int
     lib.svb_ln_patchify.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, i32, vp]
     lib.svb_head.restype = C.c_int

@@ -28,9 +28,8 @@ struct BlockParams {
     float *grn_w = nullptr, *grn_b = nullptr;  // ConvNeXt-V2: GlobalResponseNorm weight / bias [4C]; gamma is all ones then
     float* s1 = nullptr;  // LayerNorm folded into fc1 (svb_model::ln_fold): s_n = sum_k r16(W1[n,k] g_k); b1 then holds t_n
     void *w1, *w2;  // 16-bit [4C][C], [C][4C]
-    void* wdw16;    // depthwise taps as 16-bit [49][C] (the diagonal B operands of the tensor-core depthwise kernel)
     void* wtc = nullptr;  // dwconv_rawtc_kernel: [C/64][7 dy][112 = (dx, c')][64 k] 16-bit, zero except k % 16 == c' (see the kernel)
-    CUtensorMap wdw_map, wdw16_map, w1_map, w2_map, wtc_map, wtc2_map;  // wtc2: 56-row boxes (each CTA of a pair stages half of a B matrix)
+    CUtensorMap wdw_map, w1_map, w2_map, wtc_map, wtc2_map;  // wtc2: 56-row boxes (each CTA of a pair stages half of a B matrix)
     CUtensorMap w1f_map, w2f_map;  // fused-MLP weight boxes: W1 {64, 32}, W2 {64, C/2} (each CTA of the pair stages half a tile)
 };
 struct DownParams {
@@ -44,8 +43,6 @@ struct ActPlan {  // tensor maps that depend on the workspace pointer and the mi
     CUtensorMap x_map[4];   // 4-D NHWC halo maps per stage
     CUtensorMap xr_map[4];  // the same for dwconv_raw_kernel (16-pixel-wide tiles: box {64, 22, 14, 1})
     CUtensorMap xr4_map[4]; // ... and its 4-row tiles (box {64, 22, 10, 1})
-    CUtensorMap xtc_map[4]; // 4-D NHWC maps of the tensor-core depthwise kernel: box {64, W+6, rows, 1}, 128B swizzle
-    int tc_rows[4] = {0, 0, 0, 0};  // rows per box; 0 = the stage runs the CUDA-core kernel
     CUtensorMap xtc2_map[4];         // dwconv_rawtc_kernel: box {64, W, 256 / W + 6, 1} (mode A) or {64, 32, 14, 1} (mode B), 128B swizzle
     int tc2[4] = {0, 0, 0, 0};       // 0 = the stage runs dwconv_raw_kernel; 1 = mode A; 2 = mode B
     CUtensorMap a_map[4];   // [M, C]   fc1 A operand
@@ -176,41 +173,11 @@ static int gemm_cg(int N, int K) {
     return (K >= 1024 || (K >= 512 && N >= 512)) ? 2 : 1;
 }
 
-// Co-resident ("half-SM") GEMM footprint, per stage: SVB_COEX is a string of four 0/1 flags (stage 0..3), e.g. "1110".
-// A stage whose flag is set runs its fc1 / fc2 GEMMs as gemm_kernel<.., BN = 128, .., HALF = 1> (<= 113.5 KB of shared
-// memory, 256 TMEM columns), so that the other micro-batch chain's depthwise-conv CTAs fit on the same SM.
-static bool coex_stage(int s) {
-    static int mask = -1;
-    if (mask < 0) {
-        mask = 0;
-        const char* e = getenv("SVB_COEX");
-        for (int i = 0; e && i < 4 && e[i]; ++i)
-            if (e[i] == '1') mask |= 1 << i;
-    }
-    return s >= 0 && s < 4 && ((mask >> s) & 1);
-}
-// standalone svb_gemm: SVB_GEMM_HALF=1 selects the co-resident footprint (tests / experiments); read on every call
-static bool gemm_half_env() {
-    const char* e = getenv("SVB_GEMM_HALF");
-    return e && e[0] == '1';
-}
-static int gemm_bn_for(int N, bool half) { return half ? 128 : gemm_bn(N); }
 // SVB_LN_FOLD=0 (read when a model is created): keep the round-1 block -- dwconv_ln_kernel writes the NORMALISED fc1 operand,
 // fc1 is a plain bias + GELU GEMM.  Default: folded (see dwconv_raw_kernel).
 static bool ln_fold_env() {
     const char* e = getenv("SVB_LN_FOLD");
     return !(e && e[0] == '0');
-}
-// SVB_CARVEOUT=1: ask for the maximum shared-memory carve-out on the persistent kernels.  Two kernels whose preferred L1 /
-// shared split differs cannot be resident on one SM at the same time (the split is an SM-wide setting), so a half-SM GEMM
-// CTA and a depthwise CTA only ever share an SM when both ask for the same split.
-static bool carveout_max() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("SVB_CARVEOUT");
-        v = (e && e[0] == '1') ? 1 : 0;
-    }
-    return v != 0;
 }
 
 // rows per depthwise tile: bounded by the 512 TMEM columns a CTA may hold (2 warps x TH pixels x NV values), see DwCfg
@@ -240,24 +207,6 @@ static int mlp_fused_env() {
 }
 static bool mlp_fused(int setting, int C) { return setting == 1 && (C == 128 || C == 256); }          // un-folded forward: opt-in
 static bool mlp_fused_lnf(int setting, int C) { return setting != 0 && (C == 128 || C == 256); }      // folded forward: default
-// Tensor-core depthwise kernel (shifted-view diagonal MMAs): C = 256 / 512 when one stage pair of halo tiles fits
-// in shared memory.  SVB_DWCONV_TC=0 forces the CUDA-core kernel everywhere (A/B testing).
-static int dw_tc_rows(int C, int W) {
-    // Measured on B200 (profiles/r01_dwconv_tc.txt): correct, but 3x SLOWER than the FP32-pipe kernel -- every tap re-reads
-    // its 128 x 16 operand slice from shared memory (16x redundant MMAs also mean 16x redundant operand traffic), so the
-    // kernel is bound by the shared-memory operand feed, not the tensor pipe.  Kept as tested evidence; off by default.
-    static int enabled = -1;
-    if (enabled < 0) {
-        const char* e = getenv("SVB_DWCONV_TC");
-        enabled = (e && e[0] == '1') ? 1 : 0;
-    }
-    if (!enabled || (C != 256 && C != 512)) return 0;
-    const int P = W + 6;
-    const int NR = (2 * P + 132) / P + 6;
-    if (P > 256 || NR > 256) return 0;
-    const int smem = C == 512 ? DwTcCfg<512>::smem_bytes(P, NR) : DwTcCfg<256>::smem_bytes(P, NR);
-    return smem <= 227 * 1024 ? NR : 0;
-}
 
 // dwconv_rawtc_kernel (the 7 x 7 taps as seven row-shifted tcgen05 MMAs with the stencil columns in N).  0 = the stage keeps
 // dwconv_raw_kernel; 1 = mode A (W in {8, 16, 32}: units of whole image rows); 2 = mode B (32-lane windows with an x halo).
@@ -465,9 +414,6 @@ extern "C" int svb_model_create(svb_model** out, const svb_weight_desc* weights,
             for (int c = 0; c < C; ++c)
                 for (int t = 0; t < 49; ++t) taps[(size_t)t * C + c] = cw->data[(size_t)c * 49 + t];
             bp.wdw = static_cast<float*>(slab.put(taps.data(), taps.size() * 4));
-            tmp16.resize((size_t)49 * C);
-            for (size_t i = 0; i < tmp16.size(); ++i) tmp16[i] = to16(taps[i], dtype);
-            bp.wdw16 = slab.put(tmp16.data(), tmp16.size() * 2);
             if (C % 64 == 0) {  // B operands of dwconv_rawtc_kernel (98 KB per 64 channels)
                 tmp16.resize((size_t)(C / 64) * 7 * 112 * 64);
                 pack_wtc(taps.data(), tmp16.data(), C, dtype);
@@ -574,22 +520,13 @@ extern "C" int svb_model_create(svb_model** out, const svb_weight_desc* weights,
             if (m->v2) { rebase(bp.grn_w, base); rebase(bp.grn_b, base); }
             bp.w1 = base + reinterpret_cast<size_t>(bp.w1);
             bp.w2 = base + reinterpret_cast<size_t>(bp.w2);
-            bp.wdw16 = base + reinterpret_cast<size_t>(bp.wdw16);
             if (C % 64 == 0) {
                 bp.wtc = base + reinterpret_cast<size_t>(bp.wtc);
                 if (int rc = make_wtc_map(&bp.wtc_map, dtype, bp.wtc, C)) return rc;
                 if (int rc = make_wtc_map(&bp.wtc2_map, dtype, bp.wtc, C, 56)) return rc;
             }
-            {
-                const uint64_t dims16[2] = {(uint64_t)C, 49};
-                const uint64_t strides16[1] = {(uint64_t)C * 2};
-                const uint32_t box16[2] = {64, 49};
-                if (int rc = encode_tmap(&bp.wdw16_map, tmap_dtype(dtype), 2, bp.wdw16, dims16, strides16, box16,
-                                         CU_TENSOR_MAP_SWIZZLE_NONE))
-                    return rc;
-            }
-            if (int rc = make_operand_map(&bp.w1_map, dtype, bp.w1, 4 * (uint64_t)C, C, gemm_bn_for(4 * C, coex_stage(s)) / gemm_cg(4 * C, C))) return rc;
-            if (int rc = make_operand_map(&bp.w2_map, dtype, bp.w2, C, 4 * (uint64_t)C, gemm_bn_for(C, coex_stage(s)) / gemm_cg(C, 4 * C))) return rc;
+            if (int rc = make_operand_map(&bp.w1_map, dtype, bp.w1, 4 * (uint64_t)C, C, gemm_bn(4 * C) / gemm_cg(4 * C, C))) return rc;
+            if (int rc = make_operand_map(&bp.w2_map, dtype, bp.w2, C, 4 * (uint64_t)C, gemm_bn(C) / gemm_cg(C, 4 * C))) return rc;
             if (C == 128 || C == 256) {
                 if (int rc = make_operand_map(&bp.w1f_map, dtype, bp.w1, 4 * (uint64_t)C, C, 32)) return rc;
                 if (int rc = make_operand_map(&bp.w2f_map, dtype, bp.w2, C, 4 * (uint64_t)C, C / 2)) return rc;
@@ -687,15 +624,6 @@ static int build_plan(svb_model* m, ActPlan* p, uint8_t* ws, int nb, int H, int 
                                      CU_TENSOR_MAP_SWIZZLE_NONE))
                 return rc;
         }
-        p->tc_rows[s] = dw_tc_rows((int)C, w);
-        if (p->tc_rows[s]) {
-            const uint64_t dims[4] = {C, (uint64_t)w, (uint64_t)h, (uint64_t)nb};
-            const uint64_t strides[3] = {C * 2, (uint64_t)w * C * 2, (uint64_t)h * w * C * 2};
-            const uint32_t box[4] = {64, (uint32_t)(w + 6), (uint32_t)p->tc_rows[s], 1};
-            if (int rc = encode_tmap(&p->xtc_map[s], tmap_dtype(m->dtype), 4, ws + L.x, dims, strides, box,
-                                     CU_TENSOR_MAP_SWIZZLE_128B))
-                return rc;
-        }
         p->tc2[s] = m->ln_fold ? dw_tc2_mode(m->tc2_setting, m->dtype, (int)C, h, w) : 0;
         if (p->tc2[s]) {
             if (int rc = make_xtc2_map(&p->xtc2_map[s], m->dtype, ws + L.x, (int)C, nb, h, w, p->tc2[s])) return rc;
@@ -728,16 +656,15 @@ static int get_plan(svb_model* m, uint8_t* ws, int nb, int H, int W, ActPlan** o
 }
 
 // ---- launchers -------------------------------------------------------------------------------
-template <typename T, int BN, int MODE, int CG, int HALF = 0>
+template <typename T, int BN, int MODE, int CG>
 static int launch_gemm_t(const CUtensorMap& a, const CUtensorMap& w, const CUtensorMap& out, const CUtensorMap& resid,
                          const float* bias, const float* gamma, int M, int N, int K, cudaStream_t st, const float2* rowstat = nullptr, int m0 = 0) {
-    using Cfg = GemmCfg<BN, CG, HALF>;
-    auto kern = gemm_kernel<T, BN, MODE, CG, HALF>;
+    using Cfg = GemmCfg<BN, CG>;
+    auto kern = gemm_kernel<T, BN, MODE, CG>;
     static bool attr_done[MAX_DEVICES] = {};
     const int dslot = current_device_slot();
     if (!attr_done[dslot]) {
         SVB_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-        if (carveout_max()) SVB_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         attr_done[dslot] = true;
     }
     const int tiles = ceil_div(M - m0, 128 * CG) * ceil_div(N, BN);
@@ -763,25 +690,12 @@ static int launch_gemm_t(const CUtensorMap& a, const CUtensorMap& w, const CUten
 }
 template <typename T>
 static int launch_gemm(const CUtensorMap& a, const CUtensorMap& w, const CUtensorMap& out, const CUtensorMap& resid,
-                       const float* bias, const float* gamma, int M, int N, int K, int mode, cudaStream_t st, bool half = false,
+                       const float* bias, const float* gamma, int M, int N, int K, int mode, cudaStream_t st,
                        const float2* rowstat = nullptr, int m0 = 0) {
     SVB_REQUIRE(N % 32 == 0 && K % 8 == 0, SVB_ERR_INVALID_ARG, "gemm: N (%d) must be a multiple of 32, K (%d) of 8", N, K);
-    SVB_REQUIRE(mode != GEMM_LNGELU || (rowstat && gamma && !half), SVB_ERR_INVALID_ARG, "gemm: the folded-LayerNorm mode needs rowstat and s_n");
-    const int bn = gemm_bn_for(N, half);
+    SVB_REQUIRE(mode != GEMM_LNGELU || (rowstat && gamma), SVB_ERR_INVALID_ARG, "gemm: the folded-LayerNorm mode needs rowstat and s_n");
+    const int bn = gemm_bn(N);
     const int cg = gemm_cg(N, K);
-    if (half) {
-#define SVB_GEMM_HALF_CASE(MODE_, CG_)                                          \
-    if (mode == MODE_ && cg == CG_)                                             \
-        return launch_gemm_t<T, 128, MODE_, CG_, 1>(a, w, out, resid, bias, gamma, M, N, K, st, nullptr, m0);
-        SVB_GEMM_HALF_CASE(GEMM_GELU, 2)
-        SVB_GEMM_HALF_CASE(GEMM_RESID, 2)
-        SVB_GEMM_HALF_CASE(GEMM_BIAS, 2)
-        SVB_GEMM_HALF_CASE(GEMM_GELU, 1)
-        SVB_GEMM_HALF_CASE(GEMM_RESID, 1)
-        SVB_GEMM_HALF_CASE(GEMM_BIAS, 1)
-#undef SVB_GEMM_HALF_CASE
-        return set_error(SVB_ERR_INVALID_ARG, "gemm: unsupported mode %d", mode);
-    }
 #define SVB_GEMM_CASE(BN_, MODE_, CG_)                                          \
     if (bn == BN_ && mode == MODE_ && cg == CG_)                                \
         return launch_gemm_t<T, BN_, MODE_, CG_>(a, w, out, resid, bias, gamma, M, N, K, st, rowstat, m0);
@@ -857,7 +771,6 @@ static int launch_dwconv_t(const CUtensorMap& x, const BlockParams& bp, void* ou
     const int dslot = current_device_slot();
     if (!attr_done[dslot]) {
         SVB_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-        if (carveout_max()) SVB_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         attr_done[dslot] = true;
     }
     const int tx = ceil_div(W, Cfg::TW), ty = ceil_div(H, TH);
@@ -1023,32 +936,6 @@ static int launch_dwconv_raw(const CUtensorMap& x, const CUtensorMap& x4, const 
         case 2816: return launch_dwconv_raw_t<T, 2816>(x, x4, bp, out, rowstat, nb, H, W, st, b0);
     }
     return set_error(SVB_ERR_UNSUPPORTED_MODEL, "dwconv (raw): unsupported width %d", C);
-}
-template <typename T, int C>
-static int launch_dwconv_tc_t(const CUtensorMap& xtc, const BlockParams& bp, void* out, int nb, int H, int W, int NR, cudaStream_t st) {
-    using Cfg = DwTcCfg<C>;
-    auto kern = dwconv_ln_tc_kernel<T, C>;
-    const int P = W + 6;
-    const int smem = Cfg::smem_bytes(P, NR);
-    static int attr_smem[MAX_DEVICES] = {};
-    const int dslot = current_device_slot();
-    if (smem > attr_smem[dslot]) {
-        SVB_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        attr_smem[dslot] = smem;
-    }
-    const int tiles_per_img = ceil_div(H * P, 128);
-    const int tiles = nb * tiles_per_img;
-    const int grid = tiles < num_sms() ? tiles : num_sms();
-    kern<<<grid, Cfg::NUM_THREADS, smem, st>>>(xtc, bp.wdw16_map, bp.bdw, bp.lnw, bp.lnb, static_cast<T*>(out), H, W, NR,
-                                               Cfg::stage_bytes(P, NR), tiles_per_img, tiles);
-    SVB_LAUNCHED();
-    return SVB_OK;
-}
-template <typename T>
-static int launch_dwconv_tc(const CUtensorMap& xtc, const BlockParams& bp, void* out, int C, int nb, int H, int W, int NR, cudaStream_t st) {
-    if (C == 512) return launch_dwconv_tc_t<T, 512>(xtc, bp, out, nb, H, W, NR, st);
-    if (C == 256) return launch_dwconv_tc_t<T, 256>(xtc, bp, out, nb, H, W, NR, st);
-    return set_error(SVB_ERR_UNSUPPORTED_MODEL, "dwconv (tensor-core): unsupported width %d", C);
 }
 template <typename T>
 static int launch_dwconv(const CUtensorMap& x, const BlockParams& bp, void* out, int C, int nb, int H, int W, cudaStream_t st) {
@@ -1258,31 +1145,27 @@ static int forward_chunk(svb_model* m, const uint8_t* in, const float* in_f32, i
                         continue;
                     }
                     RUN(SVB_KC_GEMM, launch_gemm<T>(plan->a_map[s], bp.w1_map, plan->oh_map[s], plan->oh_map[s], bp.b1, bp.s1, m1, 4 * C, C,
-                                                    GEMM_LNGELU, st, false, rowstat, m0));
+                                                    GEMM_LNGELU, st, rowstat, m0));
                     if (m->v2) RUN(SVB_KC_GEMM, launch_grn<T>(Hd + (size_t)m0 * 4 * C, ns, tok, 4 * C, bp.grn_w, bp.grn_b,
                                                               reinterpret_cast<float*>(ws + L.grn_part), reinterpret_cast<float*>(ws + L.grn_scale), st));
                     RUN(SVB_KC_GEMM, launch_gemm<T>(plan->h_map[s], bp.w2_map, plan->ox_map[s], plan->ox_map[s], bp.b2, bp.gamma, m1, C, 4 * C,
-                                                    GEMM_RESID, st, false, nullptr, m0));
+                                                    GEMM_RESID, st, nullptr, m0));
                 }
             }
             if (int rc = stage_done(s, h, w)) return rc;
             continue;
         }
         for (const BlockParams& bp : m->blocks[s]) {
-            if (plan->tc_rows[s]) {
-                RUN(SVB_KC_DWCONV_LN, launch_dwconv_tc<T>(plan->xtc_map[s], bp, A, C, nb, h, w, plan->tc_rows[s], st));
-            } else {
-                RUN(SVB_KC_DWCONV_LN, launch_dwconv<T>(plan->x_map[s], bp, A, C, nb, h, w, st));
-            }
+            RUN(SVB_KC_DWCONV_LN, launch_dwconv<T>(plan->x_map[s], bp, A, C, nb, h, w, st));
             if (mlp_fused(m->mlp_fused_setting, C) && !m->v2) {
                 RUN(SVB_KC_MLP_FUSED, launch_mlp_fused<T>(plan->a_map[s], bp, plan->ox_map[s], C, M, st));
             } else {
                 RUN(SVB_KC_GEMM, launch_gemm<T>(plan->a_map[s], bp.w1_map, plan->oh_map[s], plan->oh_map[s], bp.b1, nullptr, M, 4 * C, C,
-                                                GEMM_GELU, st, coex_stage(s)));
+                                                GEMM_GELU, st));
                 if (m->v2) RUN(SVB_KC_GEMM, launch_grn<T>(Hd, nb, h * w, 4 * C, bp.grn_w, bp.grn_b, reinterpret_cast<float*>(ws + L.grn_part),
                                                           reinterpret_cast<float*>(ws + L.grn_scale), st));
                 RUN(SVB_KC_GEMM, launch_gemm<T>(plan->h_map[s], bp.w2_map, plan->ox_map[s], plan->ox_map[s], bp.b2, bp.gamma, M, C, 4 * C,
-                                                GEMM_RESID, st, coex_stage(s)));
+                                                GEMM_RESID, st));
             }
         }
         if (int rc = stage_done(s, h, w)) return rc;
@@ -1576,13 +1459,12 @@ extern "C" int svb_gemm(const void* d_a, const void* d_w, void* d_out, const voi
     SVB_REQUIRE(M > 0 && N > 0 && K > 0, SVB_ERR_INVALID_ARG, "gemm: bad shape");
     CUtensorMap a_map, w_map, out_map, resid_map;
     if (int rc = make_operand_map(&a_map, dtype, d_a, M, K, 128)) return rc;
-    const bool half = gemm_half_env() && N % 128 == 0 && mode != GEMM_LNGELU;
     const float2* rowstat = mode == GEMM_LNGELU ? static_cast<const float2*>(d_resid) : nullptr;
-    if (int rc = make_operand_map(&w_map, dtype, d_w, N, K, gemm_bn_for(N, half) / gemm_cg(N, K))) return rc;
+    if (int rc = make_operand_map(&w_map, dtype, d_w, N, K, gemm_bn(N) / gemm_cg(N, K))) return rc;
     if (int rc = make_epilogue_map(&out_map, dtype, d_out, M, N)) return rc;
     if (int rc = make_epilogue_map(&resid_map, dtype, mode == GEMM_RESID ? d_resid : d_out, M, N)) return rc;
-    if (dtype == SVB_FP16) return launch_gemm<__half>(a_map, w_map, out_map, resid_map, d_bias, d_gamma, M, N, K, mode, st, half, rowstat);
-    return launch_gemm<__nv_bfloat16>(a_map, w_map, out_map, resid_map, d_bias, d_gamma, M, N, K, mode, st, half, rowstat);
+    if (dtype == SVB_FP16) return launch_gemm<__half>(a_map, w_map, out_map, resid_map, d_bias, d_gamma, M, N, K, mode, st, rowstat);
+    return launch_gemm<__nv_bfloat16>(a_map, w_map, out_map, resid_map, d_bias, d_gamma, M, N, K, mode, st, rowstat);
 }
 
 extern "C" int svb_mlp_fused(const void* d_a, const void* d_w1, const float* d_b1, const void* d_w2, const float* d_b2,
@@ -1741,39 +1623,6 @@ extern "C" int svb_dwconv_raw_tc(const void* d_x, const void* d_wtc, const float
     const bool pair = (dw_tc2_env() >> 5) & 1;  // SVB_TC2_PAIR=1: the cta_group::2 variant (read per call: tests compare both)
     if (dtype == SVB_FP16) return launch_dwconv_rawtc<__half>(x_map, bp, d_out, rs, sp, C, B, H, W, mode, st, 0, true, pair);
     return launch_dwconv_rawtc<__nv_bfloat16>(x_map, bp, d_out, rs, sp, C, B, H, W, mode, st, 0, true, pair);
-}
-
-extern "C" int svb_dwconv_ln_tc(const void* d_x, const void* d_taps16, const float* d_bias, const float* d_lnw,
-                                const float* d_lnb, void* d_out, int B, int H, int W, int C, int dtype, void* stream_) {
-    cudaStream_t st = static_cast<cudaStream_t>(stream_);
-    if (int rc = check_device_sm100()) return rc;
-    SVB_REQUIRE(d_x && d_taps16 && d_bias && d_lnw && d_lnb && d_out && B > 0 && H > 0 && W > 0, SVB_ERR_INVALID_ARG,
-                "dwconv_ln_tc: bad arguments");
-    const int P = W + 6;
-    const int NR = (C == 256 || C == 512) ? (2 * P + 132) / P + 6 : 0;
-    SVB_REQUIRE(NR > 0 && (C == 512 ? DwTcCfg<512>::smem_bytes(P, NR) : DwTcCfg<256>::smem_bytes(P, NR)) <= 227 * 1024,
-                SVB_ERR_UNSUPPORTED_MODEL, "dwconv_ln_tc: C=%d W=%d is outside the tensor-core kernel's range", C, W);
-    BlockParams bp{};
-    bp.bdw = const_cast<float*>(d_bias);
-    bp.lnw = const_cast<float*>(d_lnw);
-    bp.lnb = const_cast<float*>(d_lnb);
-    {
-        const uint64_t dims[2] = {(uint64_t)C, 49};
-        const uint64_t strides[1] = {(uint64_t)C * 2};
-        const uint32_t box[2] = {64, 49};
-        if (int rc = encode_tmap(&bp.wdw16_map, tmap_dtype(dtype), 2, d_taps16, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_NONE))
-            return rc;
-    }
-    CUtensorMap x_map;
-    {
-        const uint64_t uC = C;
-        const uint64_t dims[4] = {uC, (uint64_t)W, (uint64_t)H, (uint64_t)B};
-        const uint64_t strides[3] = {uC * 2, (uint64_t)W * uC * 2, (uint64_t)H * W * uC * 2};
-        const uint32_t box[4] = {64, (uint32_t)(W + 6), (uint32_t)NR, 1};
-        if (int rc = encode_tmap(&x_map, tmap_dtype(dtype), 4, d_x, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
-    }
-    if (dtype == SVB_FP16) return launch_dwconv_tc<__half>(x_map, bp, d_out, C, B, H, W, NR, st);
-    return launch_dwconv_tc<__nv_bfloat16>(x_map, bp, d_out, C, B, H, W, NR, st);
 }
 
 extern "C" int svb_ln_patchify(const void* d_x, const float* d_lnw, const float* d_lnb, void* d_out, int B, int H, int W,

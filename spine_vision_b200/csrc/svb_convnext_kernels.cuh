@@ -810,18 +810,15 @@ dwconv_raw_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_consta
 // (rstd_m, -mu_m rstd_m) = rowstat[m], s_n passed as `gamma`, t_n as `bias`
 enum GemmMode { GEMM_GELU = 0, GEMM_RESID = 1, GEMM_BIAS = 2, GEMM_LNGELU = 3 };
 
-// HALF == 1: the "co-resident" footprint -- at most half of an SM (<= 113.5 KB of shared memory, 256 TMEM columns, 320
-// threads), so that a depthwise-conv CTA of the OTHER micro-batch chain (or a second GEMM CTA) fits beside it and the
-// FP32 pipe works under the tensor pipe's shadow.  BN = 128 only (2 accumulator stages x 128 columns).
-template <int BN, int CG, int HALF = 0>
+template <int BN, int CG>
 struct GemmCfg {
     static constexpr int BM = 128, BK = 64;
     static constexpr int B_ROWS = BN / CG;             // rows of W this CTA stages
     static constexpr int A_BYTES = BM * BK * 2;
     static constexpr int B_BYTES = B_ROWS * BK * 2;
     static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-    static constexpr int STAGES = ((HALF ? 96 : 192) * 1024) / STAGE_BYTES;  // full: 4 (48 KB), 6 (32 KB) or 8 (24 KB); half: 3 or 4
-    static constexpr int EPI_WARPS = HALF ? 8 : 16;            // 4 (2) per TMEM lane quarter: the epilogue is latency-bound per warp
+    static constexpr int STAGES = (192 * 1024) / STAGE_BYTES;  // 4 (48 KB), 6 (32 KB) or 8 (24 KB)
+    static constexpr int EPI_WARPS = 16;                       // 4 per TMEM lane quarter: the epilogue is latency-bound per warp
     static constexpr int EPI_BUF_BYTES = 32 * 32 * 2;          // one 32x32 16-bit box per warp
     static constexpr int EPI_BYTES = EPI_WARPS * EPI_BUF_BYTES;
     static constexpr int NUM_BARS = 2 * STAGES + 4 + EPI_WARPS;
@@ -830,7 +827,6 @@ struct GemmCfg {
     static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + EPI_BYTES + 512 + 1024;
     static_assert(NUM_BARS * 8 + 8 <= 512, "barrier area");
     static_assert(B_BYTES % 1024 == 0, "B stage must keep 1024-byte (swizzle atom) alignment");
-    static_assert(!HALF || (TMEM_COLS <= 256 && SMEM_BYTES <= 114 * 1024), "co-resident footprint");
 };
 
 template <typename T> struct UmmaFmt;
@@ -872,14 +868,14 @@ __device__ __forceinline__ void sts128(uint32_t addr, uint4 v) {
     asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
 }
 
-template <typename T, int BN, int MODE, int CG, int HALF = 0>
-__global__ void __launch_bounds__(GemmCfg<BN, CG, HALF>::NUM_THREADS, HALF ? 2 : 1)  // HALF: <= 102 registers, so that it fits beside a depthwise CTA
+template <typename T, int BN, int MODE, int CG>
+__global__ void __launch_bounds__(GemmCfg<BN, CG>::NUM_THREADS, 1)
 gemm_kernel(const __grid_constant__ CUtensorMap a_map, const __grid_constant__ CUtensorMap w_map,
             const __grid_constant__ CUtensorMap out_map, const __grid_constant__ CUtensorMap resid_map,
             const float* __restrict__ bias, const float* __restrict__ gamma, int M, int N, int K,
             const float2* __restrict__ rowstat, int m0) {
     // rows [m0, M) of the operands the tensor maps describe (m0 a multiple of the tile height: a sub-batch of a micro-batch)
-    using Cfg = GemmCfg<BN, CG, HALF>;
+    using Cfg = GemmCfg<BN, CG>;
     constexpr int STAGES = Cfg::STAGES;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);  // pointer arithmetic keeps the shared address space
@@ -1533,10 +1529,10 @@ mlp_fused_kernel(const __grid_constant__ CUtensorMap a_map, const __grid_constan
 
 // ============================================================================ depthwise 7x7 (raw + statistics) on the tensor cores
 // dwconv_raw_kernel's contract (raw 16-bit convolution = the fc1 A operand, (rstd, -mu rstd) per token) with the 49 taps on the
-// tensor pipe.  The first tensor-core version (dwconv_ln_tc_kernel below) issued one MMA per TAP and was bound by the operand
-// feed: each 128 x 16 activation slice was re-read from shared memory 49 times.  Here a slice is read SEVEN times:
+// tensor pipe.  One MMA per TAP (16 x 16 diagonal B matrices) is bound by the operand feed: each 128 x 16 activation slice is
+// re-read from shared memory 49 times (measured and rejected, DESIGN.md).  Here a slice is read SEVEN times:
 //   * the seven ROWS of the stencil (dy) are seven accumulating MMAs over row-shifted views of one swizzled tile (a row of 32
-//     lanes is 4 KB, so every view starts on a 1024-byte swizzle atom);
+//     lanes is 4 KB, so every view starts on a 1024-byte swizzle atom; scripts/ubench/shiftmma.cu checks shifted views);
 //   * the seven COLUMNS (dx) sit side by side in the N dimension: B_dy[k = c, n = (dx, c')] = w[dy][dx][c] (c == c'), 0 otherwise,
 //     an M = 128, N = 7 x 16 = 112, K = 16 MMA per 16 channels, so TMEM lane p (a SOURCE pixel) ends up holding
 //         D[p][dx][c] = sum_dy in[y(p) + dy - 3, x(p), c] * w[dy][dx][c]
@@ -1886,292 +1882,6 @@ __global__ void __launch_bounds__(256) ln_stat_finalize_kernel(const float2* __r
     const float var = fmaxf(fmaf(-mu, mu, sq * inv_c), 0.0f);
     const float rstd = 1.0f / sqrtf(var + LN_EPS_BACKBONE);
     rowstat[t] = make_float2(rstd, -mu * rstd);
-}
-
-// ============================================================================ depthwise 7x7 + LayerNorm on the tensor cores
-// The 49-tap depthwise convolution is run as tcgen05 MMAs over SHIFTED VIEWS of one shared-memory halo tile:
-// the (zero-padded) image rows of a 64-channel chunk sit in shared memory as 128-byte pixel rows (TMA,
-// SWIZZLE_128B, padded row pitch P = W + 6), so the 128 consecutive padded-linear output pixels p0..p0+127 read,
-// for tap (ky,kx), the 128 consecutive pixel rows starting at p0 + ky*P + kx -- one K-major A operand whose start
-// address is simply moved by whole rows (the 128B swizzle is a function of the absolute shared-memory address,
-// so any row offset is a valid operand start; verified on B200, scripts/ubench/shiftmma.cu).  Per tap and per 16
-// channels the B operand is the 16x16 diagonal matrix of that tap's weights, so
-//     D[128 px, 16 ch] += A_shift(ky,kx)[128 px, 16 ch] * diag(w[ky][kx][16 ch])
-// is one M=128, N=16, K=16 MMA: 16x redundant arithmetic, which the tensor pipe (4096 MAC/clk/SM) still finishes
-// ~3x sooner than the FP32 pipe (128 FMA/clk/SM peak, ~65 achieved) does the useful 1/16.  Accumulators for all C
-// channels of the 128 pixels live in TMEM (C fp32 columns), so LayerNorm over C is per-thread (lane = pixel).
-//   warp 0        TMA producer: halo tile + the chunk's 49x64 16-bit taps per stage
-//   warp 1        MMA issuer (one lane): 49 taps x 4 channel blocks per chunk
-//   warp 2        diagonal-B generator: writes the 16 diagonal entries of each (tap, block) matrix into a zeroed ring
-//   warps 4..19   epilogue: bias + LayerNorm statistics (Chan-merged per 32-column pass), normalise, 16-bit store;
-//                 columns are handed back to the MMA issuer chunk by chunk, so the next tile's MMAs start while this
-//                 tile is still being written out.
-template <int C>
-struct DwTcCfg {
-    static constexpr int CC = 64, NCH = C / CC;
-    static constexpr int A_STAGES = 2;
-    static constexpr int TAP_BYTES = 49 * CC * 2;                 // the chunk's taps, 16-bit, [49][64]
-    static constexpr int B_BLOCK = 512;                           // one 16x16 16-bit matrix (4 core matrices)
-    static constexpr int B_SLOT = 7 * 4 * B_BLOCK;                // one ky row of taps x 4 channel blocks
-    static constexpr int B_SLOTS = 3;
-    static constexpr int EPI_WARPS = 16;
-    static constexpr int EPI_BUF = 32 * 64;                       // 32 pixels x 32 channels, 16-bit
-    static constexpr int NUM_THREADS = 32 * (4 + EPI_WARPS);
-    static constexpr int NUM_BARS = 2 * A_STAGES + 2 * B_SLOTS + 1 + NCH;
-    static constexpr int TMEM_COLS = C;                           // 128 / 256 / 512
-    static_assert(C == 256 || C == 512, "one fp32 TMEM column per channel (C <= 512); each epilogue warp owns whole 64-column chunks (C >= 256)");
-    static int stage_bytes(int P, int NR) { return (int)align_up((size_t)NR * P * 128 + TAP_BYTES, 1024); }
-    static int smem_bytes(int P, int NR) {
-        return A_STAGES * stage_bytes(P, NR) + B_SLOTS * B_SLOT + EPI_WARPS * EPI_BUF + 128 * 4 * 8 + NUM_BARS * 8 + 64 + 1024;
-    }
-    static int rows_per_box(int P) { return (P + 133 + P - 1) / P + 6; }  // padded rows an M tile can touch
-};
-
-// no-swizzle K-major descriptor for the 16x16 diagonal B block: core matrices (n_hi, k_hi) at n_hi*256 + k_hi*128
-__device__ __forceinline__ uint64_t make_diag_b_desc(uint32_t smem_addr) {
-    uint64_t d = 0;
-    d |= static_cast<uint64_t>((smem_addr >> 4) & 0x3FFFu);
-    d |= static_cast<uint64_t>(128 >> 4) << 16;  // LBO: K-adjacent core matrices
-    d |= static_cast<uint64_t>(256 >> 4) << 32;  // SBO: N-adjacent core matrices
-    d |= static_cast<uint64_t>(1) << 46;
-    return d;
-}
-
-template <typename T, int C>
-__global__ void __launch_bounds__(DwTcCfg<C>::NUM_THREADS, 1)
-dwconv_ln_tc_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_constant__ CUtensorMap w_map,
-                    const float* __restrict__ bdw, const float* __restrict__ lnw, const float* __restrict__ lnb,
-                    T* __restrict__ out, int H, int W, int NR, int stage_bytes, int tiles_per_img, int num_tiles) {
-    using Cfg = DwTcCfg<C>;
-    constexpr int NCH = Cfg::NCH, CC = Cfg::CC;
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-    uint8_t* sA = smem;                                                   // A_STAGES x stage_bytes (halo tile, then taps)
-    uint8_t* sB = sA + Cfg::A_STAGES * stage_bytes;                       // B_SLOTS x B_SLOT
-    uint8_t* sE = sB + Cfg::B_SLOTS * Cfg::B_SLOT;                        // EPI_WARPS x EPI_BUF
-    float2* sStat = reinterpret_cast<float2*>(sE + Cfg::EPI_WARPS * Cfg::EPI_BUF);  // [4 slices][128 px] (mean, M2)
-    uint64_t* bars = reinterpret_cast<uint64_t*>(sStat + 4 * 128);
-    uint64_t* afull = bars;
-    uint64_t* aempty = afull + Cfg::A_STAGES;
-    uint64_t* bfull = aempty + Cfg::A_STAGES;
-    uint64_t* bempty = bfull + Cfg::B_SLOTS;
-    uint64_t* dfull = bempty + Cfg::B_SLOTS;
-    uint64_t* dfree = dfull + 1;                                          // [NCH] 64-column blocks handed back by the epilogue
-    uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(dfree + NCH);
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int P = W + 6;
-    const int tap_off = NR * P * 128;  // the taps follow the halo tile inside a stage
-
-    if (tid == 0) {
-        tma_prefetch_desc(&x_map);
-        tma_prefetch_desc(&w_map);
-        for (int s = 0; s < Cfg::A_STAGES; ++s) { mbar_init(&afull[s], 1); mbar_init(&aempty[s], 1); }
-        for (int s = 0; s < Cfg::B_SLOTS; ++s) { mbar_init(&bfull[s], 1); mbar_init(&bempty[s], 1); }
-        mbar_init(dfull, 1);
-        for (int k = 0; k < NCH; ++k) mbar_init(&dfree[k], 4);
-        mbar_fence_init();
-    }
-    if (warp == 1) tmem_alloc<1>(tmem_ptr, Cfg::TMEM_COLS);
-    // the diagonal-B ring starts out all zero; only the 16 diagonal entries of a block are ever rewritten
-    for (int i = tid; i < Cfg::B_SLOTS * Cfg::B_SLOT / 16; i += Cfg::NUM_THREADS) reinterpret_cast<uint4*>(sB)[i] = make_uint4(0, 0, 0, 0);
-    fence_proxy_async();
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_ptr;
-
-    if (warp == 0) {
-        // ------------------------------------------------------------------ TMA producer
-        if (lane == 0) {
-            int it = 0;
-            for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-                const int b = tile / tiles_per_img, p0 = (tile - b * tiles_per_img) * 128;
-                const int r0 = p0 / P;  // first padded row of the tile
-                for (int k = 0; k < NCH; ++k, ++it) {
-                    const int stage = it % Cfg::A_STAGES;
-                    if (it >= Cfg::A_STAGES) mbar_wait(&aempty[stage], ((it / Cfg::A_STAGES) - 1) & 1);
-                    uint8_t* dst = sA + stage * stage_bytes;
-                    mbar_expect_tx(&afull[stage], (uint32_t)(tap_off + Cfg::TAP_BYTES));
-                    tma_load_4d(dst, &x_map, &afull[stage], k * CC, -3, r0 - 3, b);
-                    tma_load_2d(dst + tap_off, &w_map, &afull[stage], k * CC, 0);
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ------------------------------------------------------------------ MMA issuer
-        if (lane == 0) {
-            constexpr uint32_t idesc = (1u << 4) | (UmmaFmt<T>::v << 7) | (UmmaFmt<T>::v << 10) | ((uint32_t)(16 >> 3) << 17) |
-                                       ((uint32_t)(128 >> 4) << 24);
-            int it = 0, bs = 0;
-            uint32_t bphase = 0, tcount = 0;
-            for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++tcount) {
-                const int b = tile / tiles_per_img, p0 = (tile - b * tiles_per_img) * 128;
-                const int poff = p0 - (p0 / P) * P;  // tile start inside its first padded row
-                for (int k = 0; k < NCH; ++k, ++it) {
-                    const int stage = it % Cfg::A_STAGES;
-                    if (tcount > 0) mbar_wait(&dfree[k], (tcount - 1) & 1);  // the previous tile's columns of this chunk were read out
-                    mbar_wait(&afull[stage], (it / Cfg::A_STAGES) & 1);
-                    tc_fence_after();
-                    const uint64_t a0 = make_sw128_kmajor_desc(smem_u32(sA + stage * stage_bytes) + (uint32_t)poff * 128u);
-                    const uint32_t d0 = tmem_base + (uint32_t)(k * CC);
-                    for (int ky = 0; ky < 7; ++ky) {
-                        mbar_wait(&bfull[bs], bphase);
-                        tc_fence_after();
-                        const uint64_t b0 = make_diag_b_desc(smem_u32(sB + bs * Cfg::B_SLOT));
-                        const uint64_t arow = a0 + (uint64_t)((ky * P) * 8);  // 128 B per pixel row = 8 descriptor units
-#pragma unroll
-                        for (int kx = 0; kx < 7; ++kx) {
-#pragma unroll
-                            for (int blk = 0; blk < 4; ++blk)
-                                tc_mma_f16<1>(d0 + (uint32_t)(blk * 16), arow + (uint64_t)(kx * 8 + blk * 2),
-                                              b0 + (uint64_t)((kx * 4 + blk) * (Cfg::B_BLOCK >> 4)), idesc, (ky | kx) != 0 ? 1u : 0u);
-                        }
-                        tc_commit<1>(&bempty[bs]);
-                        if (++bs == Cfg::B_SLOTS) { bs = 0; bphase ^= 1; }
-                    }
-                    tc_commit<1>(&aempty[stage]);
-                }
-                tc_commit<1>(dfull);
-            }
-        }
-    } else if (warp == 2) {
-        // ------------------------------------------------------------------ diagonal-B generator
-        int it = 0, bs = 0;
-        uint32_t bphase = 0;
-        // lane -> channels lane and lane + 32 of the chunk: block (c >> 4), diagonal position n = c & 15
-        const int n = lane & 15;
-        const uint32_t diag_off = (uint32_t)((n >> 3) * 384 + (n & 7) * 18);
-        const uint32_t blk_a = (uint32_t)(lane >> 4), blk_b = blk_a + 2;
-        for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-            for (int k = 0; k < NCH; ++k, ++it) {
-                const int stage = it % Cfg::A_STAGES;
-                mbar_wait(&afull[stage], (it / Cfg::A_STAGES) & 1);
-                const uint16_t* taps = reinterpret_cast<const uint16_t*>(sA + stage * stage_bytes + tap_off);  // [49][64]
-                for (int ky = 0; ky < 7; ++ky) {
-                    mbar_wait(&bempty[bs], bphase ^ 1);
-                    uint8_t* slot = sB + bs * Cfg::B_SLOT;
-#pragma unroll
-                    for (int kx = 0; kx < 7; ++kx) {
-                        const uint16_t wa = taps[(ky * 7 + kx) * CC + lane], wb = taps[(ky * 7 + kx) * CC + lane + 32];
-                        *reinterpret_cast<uint16_t*>(slot + (kx * 4 + blk_a) * Cfg::B_BLOCK + diag_off) = wa;
-                        *reinterpret_cast<uint16_t*>(slot + (kx * 4 + blk_b) * Cfg::B_BLOCK + diag_off) = wb;
-                    }
-                    fence_proxy_async();
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive(&bfull[bs]);
-                    if (++bs == Cfg::B_SLOTS) { bs = 0; bphase ^= 1; }
-                }
-            }
-        }
-    } else if (warp >= 4) {
-        // ------------------------------------------------------------------ epilogue: bias + LayerNorm + store
-        const int ew = warp - 4;
-        const int q = warp & 3;          // TMEM lane quarter = pixels q*32 .. q*32+31 of the tile
-        const int slice = ew >> 2;       // columns slice*CW .. +CW
-        constexpr int CW = C / 4, NP = CW / 32;  // 32-column passes per warp
-        const uint32_t tbase = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(slice * CW);
-        uint8_t* ebuf = sE + ew * Cfg::EPI_BUF;
-        const uint32_t ebuf_a = smem_u32(ebuf);
-        const int px = q * 32 + lane;
-        uint32_t tcount = 0;
-        for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++tcount) {
-            const int b = tile / tiles_per_img, p0 = (tile - b * tiles_per_img) * 128;
-            const int p = p0 + px;
-            const int y = p / P, x = p - y * P;
-            const bool valid = x < W && y < H;
-            const long long tok = ((long long)b * H + y) * W + x;
-            mbar_wait(dfull, tcount & 1);
-            tc_fence_after();
-            // ---- pass 1: statistics of (acc + bias) over this warp's columns, merged 32 at a time (Chan)
-            float mean = 0.f, m2 = 0.f;
-#pragma unroll
-            for (int c4 = 0; c4 < NP; ++c4) {
-                float v[32];
-                TmemLd<32>::ld(tbase + (uint32_t)(c4 * 32), v);
-                tmem_ld_wait();
-                const float4* bp = reinterpret_cast<const float4*>(bdw + slice * CW + c4 * 32);
-                float s = 0.f;
-#pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    const float4 bb = __ldg(bp + j);
-                    v[4 * j] += bb.x; v[4 * j + 1] += bb.y; v[4 * j + 2] += bb.z; v[4 * j + 3] += bb.w;
-                    s += (v[4 * j] + v[4 * j + 1]) + (v[4 * j + 2] + v[4 * j + 3]);
-                }
-                const float mb = s * (1.0f / 32.0f);
-                float qb = 0.f;
-#pragma unroll
-                for (int j = 0; j < 32; ++j) { const float d = v[j] - mb; qb = fmaf(d, d, qb); }
-                const float na = (float)(c4 * 32), nt = (float)(c4 * 32 + 32);
-                const float delta = mb - mean;
-                mean = fmaf(delta, 32.0f / nt, mean);
-                m2 = m2 + qb + delta * delta * (na * 32.0f / nt);
-            }
-            sStat[slice * 128 + px] = make_float2(mean, m2);
-            asm volatile("bar.sync 1, %0;" ::"n"(Cfg::EPI_WARPS * 32) : "memory");
-            {
-                float2 s0 = sStat[px];
-                float nacc = (float)CW;
-#pragma unroll
-                for (int s = 1; s < 4; ++s) {
-                    const float2 sb = sStat[s * 128 + px];
-                    const float nt = nacc + (float)CW;
-                    const float delta = sb.x - s0.x;
-                    s0.x = fmaf(delta, (float)CW / nt, s0.x);
-                    s0.y = s0.y + sb.y + delta * delta * (nacc * (float)CW / nt);
-                    nacc = nt;
-                }
-                mean = s0.x;
-                m2 = s0.y;
-            }
-            const float rstd = 1.0f / sqrtf(m2 * (1.0f / C) + LN_EPS_BACKBONE);
-            asm volatile("bar.sync 2, %0;" ::"n"(Cfg::EPI_WARPS * 32) : "memory");  // sStat may be rewritten by the next tile
-            // ---- pass 2: normalise, stage 32 px x 32 ch through shared memory, write whole 64-byte row segments
-            const uint32_t row_off = ebuf_a + (uint32_t)lane * 64u;
-            const uint32_t swz = ((uint32_t)lane >> 1) & 3u;
-#pragma unroll
-            for (int c4 = 0; c4 < NP; ++c4) {
-                float v[32];
-                TmemLd<32>::ld(tbase + (uint32_t)(c4 * 32), v);
-                tmem_ld_wait();
-                const int col = slice * CW + c4 * 32;
-                if ((c4 & 1) == 1) {  // both 32-column halves of a 64-column MMA chunk are in registers / written: hand it back
-                    tc_fence_before();
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive(&dfree[col >> 6]);
-                }
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    const float4* bp = reinterpret_cast<const float4*>(bdw + col + 8 * i);
-                    const float4* wp = reinterpret_cast<const float4*>(lnw + col + 8 * i);
-                    const float4* gp = reinterpret_cast<const float4*>(lnb + col + 8 * i);
-                    uint32_t o[4];
-#pragma unroll
-                    for (int h = 0; h < 2; ++h) {
-                        const float4 bb = __ldg(bp + h), gw = __ldg(wp + h), gb = __ldg(gp + h);
-                        const int j = 8 * i + 4 * h;
-                        o[2 * h] = Cvt<T>::pack2(fmaf((v[j] + bb.x - mean) * rstd, gw.x, gb.x), fmaf((v[j + 1] + bb.y - mean) * rstd, gw.y, gb.y));
-                        o[2 * h + 1] = Cvt<T>::pack2(fmaf((v[j + 2] + bb.z - mean) * rstd, gw.z, gb.z), fmaf((v[j + 3] + bb.w - mean) * rstd, gw.w, gb.w));
-                    }
-                    sts128(row_off + ((((uint32_t)i) ^ swz) << 4), make_uint4(o[0], o[1], o[2], o[3]));
-                }
-                __syncwarp();
-                // transposed read: 8 pixels x 64 bytes per instruction
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    const int pj = (lane >> 2) + 8 * i, piece = lane & 3;
-                    const long long tj = __shfl_sync(0xffffffffu, tok, pj);
-                    const int vj = __shfl_sync(0xffffffffu, (int)valid, pj);
-                    const uint4 val = lds128(ebuf_a + (uint32_t)pj * 64u + ((((uint32_t)piece) ^ (((uint32_t)pj >> 1) & 3u)) << 4));
-                    if (vj) *reinterpret_cast<uint4*>(out + (size_t)tj * C + col + piece * 8) = val;
-                }
-                __syncwarp();
-            }
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) tmem_dealloc<1>(tmem_base, Cfg::TMEM_COLS);
 }
 
 // ============================================================================ Global Response Normalization (ConvNeXt-V2)

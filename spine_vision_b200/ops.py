@@ -607,17 +607,6 @@ def dwconv_raw_tc(x: torch.Tensor, wtc: torch.Tensor, bias: torch.Tensor, out: t
 
 
 @_on_device
-def dwconv_ln_tc(x: torch.Tensor, taps: torch.Tensor, bias: torch.Tensor, lnw: torch.Tensor, lnb: torch.Tensor):
-    """Same operator as ``dwconv_ln`` on the tensor cores (taps are rounded to the activation dtype)."""
-    B, H, W, Cc = x.shape
-    out = torch.empty_like(x)
-    taps16 = taps.to(x.dtype).contiguous()
-    _lib.check(_lib.load().svb_dwconv_ln_tc(x.data_ptr(), taps16.data_ptr(), bias.data_ptr(), lnw.data_ptr(), lnb.data_ptr(),
-                                            out.data_ptr(), B, H, W, Cc, _dt(x), _lib.current_stream()))
-    return out
-
-
-@_on_device
 def ln_patchify(x: torch.Tensor, lnw: torch.Tensor, lnb: torch.Tensor):
     B, H, W, Cc = x.shape
     out = torch.empty((B, H // 2, W // 2, 4 * Cc), dtype=x.dtype, device=x.device)
